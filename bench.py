@@ -169,6 +169,29 @@ def parity_sample(kind, results, step_pairs, raw, n_feat, row_bytes, np_dtype, c
             "checker": "oracle.match (oracle/bf_oracle.c) on the last timed device-resident step; SURF tolerance 1e-5 relative"}
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, results, step_pairs, n_feat):
+    """Writes what the caller of the timed path receives for one step as float32 .npy files (indices stay below 2^24, so they are
+    exact): pairs [P, 2] (query frame, train frame) and match_counts [P] of every pair, and the matches of a seeded sample of the
+    pairs (sample [S]: positions in the step, ascending; query_idx, train_idx, distance: their matches back to back in sample
+    order).  The sample is sized for n_feat matches per pair, the most a cross-checked 2-NN can return, so which pairs are
+    written depends only on the arguments and the files stay under DUMP_BYTES."""
+    results.fetch()
+    matches, off = results.all_matches()
+    n_pairs = len(step_pairs)
+    assert results.n_pairs == n_pairs
+    n_sample = min(n_pairs, (DUMP_BYTES - 12 * n_pairs - 1024) // (12 * n_feat + 4))
+    sample = np.sort(np.random.default_rng(2024).choice(n_pairs, n_sample, replace=False))
+    picked = np.concatenate([matches[off[k]:off[k + 1]] for k in sample]) if n_sample else matches[:0]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"pairs": step_pairs, "match_counts": np.diff(off), "sample": sample,
+              "query_idx": picked["queryIdx"], "train_idx": picked["trainIdx"], "distance": picked["distance"]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float32))
+
+
 def run_reference(args, kind):
     """--impl reference: cv2.BFMatcher on the box's host cores; rank 0 only."""
     rank = int(os.environ.get("RANK", "0"))
@@ -226,8 +249,9 @@ def workload_config(kind, pairs_per_step, e2e_frames):
     return cfg
 
 
-def bench_kind(args, kind, ctx, dev, rank, world, dist, steps, warmup, cpu_budget_s, engine=None, e2e_arm=True):
-    """Returns the result dict for one descriptor kind (device-resident value, e2e, roofline, cpu baseline).
+def bench_kind(args, kind, ctx, dev, rank, world, dist, steps, warmup, cpu_budget_s, engine=None, e2e_arm=True, dump_dir=None):
+    """Returns the result dict for one descriptor kind (device-resident value, e2e, roofline, cpu baseline); with `dump_dir`,
+    rank 0 also writes the last timed device-resident step's matches there (dump_outputs).
     `engine` selects the sweep kernel: SURF 'tc16' (tcgen05 FP16 split, slice keys) | 'tc' (tcgen05 3xTF32) | 'ffma' (exact-FP32 FMA pipe);
     ORB 'tc16' (tcgen05 FP8 dot product, FP16 accumulators, slice keys) | 'tc' (FP8 dot product delivering packed keys) | 'popc' (XOR + POPC);
     None = library default (tc16)."""
@@ -340,6 +364,8 @@ def bench_kind(args, kind, ctx, dev, rank, world, dist, steps, warmup, cpu_budge
     parity = None
     if rank == 0 and not args.no_parity:
         parity = parity_sample(kind, r_last, step_pairs(warmup + steps - 1), raw, n_feat, row_bytes, np_dtype, cols, args.parity_pairs)
+    if rank == 0 and dump_dir:
+        dump_outputs(dump_dir, r_last, step_pairs(warmup + steps - 1), n_feat)
     r_last.close()
 
     # ---- end-to-end arm: PAGEABLE host frames in, host matches out (on rank 0), through the public API -----------------
@@ -418,9 +444,9 @@ def bench_kind(args, kind, ctx, dev, rank, world, dist, steps, warmup, cpu_budge
                 return time.perf_counter() - t0
             for s in range(2):
                 pinned_step(s)
-            tp = sum(pinned_step(warmup + s) for s in range(3))
-            e2e["e2e_pinned"] = {"value": 3.0 * e2e_pairs * n_feat * n_feat / tp, "unit": "comparisons/s", "ms_per_step": 1e3 * tp / 3,
-                                 "note": "esfm_bank_set_frame_pinned (host wall clock, 3 steps)"}
+            tp = sum(pinned_step(warmup + s) for s in range(steps))
+            e2e["e2e_pinned"] = {"value": steps * e2e_pairs * n_feat * n_feat / tp, "unit": "comparisons/s", "ms_per_step": 1e3 * tp / steps,
+                                 "note": f"esfm_bank_set_frame_pinned (host wall clock, {steps} steps)"}
             del pin, pin_np
 
     # ---- roofline of the dominant kernel (the sweep) -----------------------------------------------------
@@ -583,7 +609,11 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle check of a sample of the timed step (runs under ncu)")
     ap.add_argument("--parity-pairs", type=int, default=20)
     ap.add_argument("--e2e-frames", type=int, default=0, help="frames of the fixed e2e triangle (default: ~4 x pairs_per_step pairs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline kind's last timed device-resident step (rank 0's pairs) as DIR/<name>.npy, float32, < 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -618,18 +648,19 @@ def main():
     other_engine = {"surf": {"tc16": "ffma", "tc": "ffma", "ffma": "tc16"}, "orb": {"tc16": "popc", "tc": "popc", "popc": "tc16"}}
 
     def alt_run(kind):
-        # the other engine of this kind on the same workload, device-resident arm only (short: it is context, not the headline)
-        a = bench_kind(args, kind, ctx, dev, rank, world, dist, 3, 3, 0.0, engine=other_engine[kind][engines[kind]], e2e_arm=False)
+        # the other engine of this kind on the same workload, device-resident arm only (context, not the headline)
+        a = bench_kind(args, kind, ctx, dev, rank, world, dist, args.steps, args.warmup, 0.0, engine=other_engine[kind][engines[kind]],
+                       e2e_arm=False)
         (ctx.set_l2_engine if kind == "surf" else ctx.set_hamming_engine)(engines[kind])
         return {k: a[k] for k in ("engine", "value", "unit", "ms_per_step", "roofline", "clocks", "parity_sample")}
 
     primary = bench_kind(args, args.kind, ctx, dev, rank, world, dist, args.steps, args.warmup, args.cpu_budget_s,
-                         engine=engines[args.kind])
+                         engine=engines[args.kind], dump_dir=args.dump_outputs)
     if not args.no_alt_engine and world == 1:
         primary["alt_engine"] = alt_run(args.kind)
     if not args.no_secondary:
         other = "orb" if args.kind == "surf" else "surf"
-        sec = bench_kind(args, other, ctx, dev, rank, world, dist, max(3, args.steps // 2), args.warmup, args.cpu_budget_s / 2,
+        sec = bench_kind(args, other, ctx, dev, rank, world, dist, args.steps, args.warmup, args.cpu_budget_s / 2,
                          engine=engines[other])
         primary["secondary"] = {k: sec[k] for k in ("value", "unit", "ms_per_step", "dtype", "config", "pairs_per_s", "e2e", "parity_sample",
                                                     "engine", "roofline", "cpu_baseline", "gpu_launches", "clocks", "full_job_estimate_s")}

@@ -8,7 +8,8 @@ Outputs (all small, all committed):
   synth_surf.npz      4 SURF-like frames (seeded), cv2 matches for ratio {0.5, 0.8} x cross_check {0, 1}, all 6 pairs
   synth_orb.npz       4 ORB-like frames (seeded), same grid
   fountain_orb.npz    BASELINE configs[0] stand-in: ORB_create(8000) descriptors of the 11 bundled fountain images
-                      (SURF is not in this image's OpenCV, SURVEY.md F9) + cv2 matches of all 55 pairs, cross_check 0/1
+                      (SURF is not in this image's OpenCV, SURVEY.md F9) + cv2 matches of all 55 pairs, cross_check 0/1;
+                      about 2 MB, so stored as fountain_orb.part<k>.npz (save_parts) and loaded as one by golden_util.load
 The fixtures store descriptors AND expected matches, so the tests need neither cv2 nor /root/reference.
 """
 import os
@@ -38,6 +39,23 @@ def all_pairs_expected(frames, ratios, out, prefix):
                     ij, d = pack_matches(m)
                     out[f"{prefix}_r{int(ratio * 100)}_c{cc}_{i}_{j}_idx"] = ij
                     out[f"{prefix}_r{int(ratio * 100)}_c{cc}_{i}_{j}_dist"] = d
+
+
+PART_BYTES = 900_000
+
+
+def save_parts(stem, arrays):
+    """Writes `arrays` as stem.part0.npz, stem.part1.npz, ... (compressed, in insertion order), each holding at most PART_BYTES of
+    array data so every committed file stays under 1 MB; tests/golden_util.load(stem + ".npz") merges them back."""
+    parts, size = [{}], 0
+    for k, a in arrays.items():
+        if parts[-1] and size + a.nbytes > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = a
+        size += a.nbytes
+    for n, p in enumerate(parts):
+        np.savez_compressed(f"{stem}.part{n}.npz", **p)
 
 
 def kat_cases():
@@ -111,7 +129,7 @@ def main():
         frames.append(np.ascontiguousarray(desc))
     out = {f"frame_{i}": f for i, f in enumerate(frames)}
     all_pairs_expected(frames, (0.8,), out, "m")
-    np.savez_compressed(os.path.join(HERE, "fountain_orb.npz"), **out)
+    save_parts(os.path.join(HERE, "fountain_orb"), out)
     print("fountain frames:", [f.shape[0] for f in frames])
     for f in os.listdir(HERE):
         if f.endswith(".npz"):

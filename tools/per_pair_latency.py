@@ -1,5 +1,5 @@
 """Latency of the UNMODIFIED caller's shape (sfm.cpp:153,156: one matchFeaturesX call per image pair = esfm_match_descriptors):
-config 1, the 11 bundled fountain images as ORB(8000) descriptors (tests/golden/fountain_orb.npz), 55 pairs in loop order, against
+config 1, the 11 bundled fountain images as ORB(8000) descriptors (tests/golden/fountain_orb.part*.npz), 55 pairs in loop order, against
 one esfm_match_all_pairs over the same frames.  usage: python tools/per_pair_latency.py  -> one JSON line"""
 import json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
