@@ -48,6 +48,7 @@ class Stats(ctypes.Structure):
         ("last_finalize_ms", c_double),
         ("sweep_ms_total", c_double),
         ("sweep_launches", c_uint64),
+        ("fallback_rows", c_uint64),
     ]
 
     def as_dict(self):

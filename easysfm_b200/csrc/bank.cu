@@ -114,10 +114,13 @@ cudaError_t launch_pack_tc(const float* rows, const int* frame_rows, const int* 
 // F32X64 -> the 16-bit split ("H") images of tc_layout.cuh for sweep_win.cu: per 128-row tile 16 groups x 2048 B = [a k0..63][b k0..63]
 // SWIZZLE_128B atoms of fp16 (a = fp16(x), b = fp16(x - a)) + the same 16 x 256 B augmented TF32 columns as the 3xTF32 image.
 // One block per tile, one thread per (row, 8 dims = one 16-byte chunk of each atom); byte-for-byte tch_pack_row_host.
+// Also the two inputs of win_fast_eps: per row |x - fp16(x)|_2 (the rounding of the sweep's query writers) and per frame the largest
+// |x|_2 (frame_norm must be zero on entry), both rounded up.
 __global__ void __launch_bounds__(256) pack_tch_kernel(const float* __restrict__ rows, const int* __restrict__ frame_rows,
                                                        const int* __restrict__ frame_row_off,
                                                        const int* __restrict__ frame_tile_off, int n_frames,
-                                                       unsigned char* __restrict__ tc_main) {
+                                                       unsigned char* __restrict__ tc_main, float* __restrict__ row_eps,
+                                                       float* __restrict__ frame_norm) {
     __shared__ float tile[kTile][kDim + 4];
     const int t = blockIdx.x;
     int lo = 0, hi = n_frames - 1;
@@ -151,9 +154,18 @@ __global__ void __launch_bounds__(256) pack_tch_kernel(const float* __restrict__
     __syncthreads();
     if (threadIdx.x < kTile) {
         const int r = threadIdx.x;
-        float s = 0.f;
+        float s = 0.f, se = 0.f;
 #pragma unroll 8
-        for (int k = 0; k < kDim; ++k) s = __fmaf_rn(tile[r][k], tile[r][k], s);
+        for (int k = 0; k < kDim; ++k) {
+            const float x = tile[r][k], d = x - tch_h2f(tch_f2h(x));     // exact in fp32
+            s = __fmaf_rn(x, x, s);
+            se = __fmaf_rn(d, d, se);
+        }
+        if (r < valid) {
+            // (64 fused steps: relative error < 2^-18 on the sums, the square roots are rounded up)
+            row_eps[frame_row_off[f] + row0 + r] = __fsqrt_ru(se) * (1.f + 0x1p-16f);
+            atomicMax(reinterpret_cast<int*>(frame_norm + f), __float_as_int(__fsqrt_ru(s) * (1.f + 0x1p-16f)));
+        }
         const float h = (r < valid) ? 0.5f * s : kTcPadNorm;
         float hh, hm, hl;
         tc_split3(h, hh, hm, hl);
@@ -164,9 +176,11 @@ __global__ void __launch_bounds__(256) pack_tch_kernel(const float* __restrict__
 }
 
 cudaError_t launch_pack_tch(const float* rows, const int* frame_rows, const int* frame_row_off, const int* frame_tile_off,
-                            int n_frames, int n_tiles_total, unsigned char* tc_main, cudaStream_t s) {
+                            int n_frames, int n_tiles_total, unsigned char* tc_main, float* row_eps, float* frame_norm, cudaStream_t s) {
     if (n_tiles_total <= 0) return cudaSuccess;
-    pack_tch_kernel<<<n_tiles_total, 256, 0, s>>>(rows, frame_rows, frame_row_off, frame_tile_off, n_frames, tc_main);
+    cudaError_t e = cudaMemsetAsync(frame_norm, 0, (size_t)n_frames * sizeof(float), s);
+    if (e != cudaSuccess) return e;
+    pack_tch_kernel<<<n_tiles_total, 256, 0, s>>>(rows, frame_rows, frame_row_off, frame_tile_off, n_frames, tc_main, row_eps, frame_norm);
     return cudaGetLastError();
 }
 

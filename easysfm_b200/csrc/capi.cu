@@ -259,6 +259,7 @@ extern "C" int esfm_init(int device, void* cuda_stream, esfm_ctx_t** out) {
     ctx->sm_count = prop.multiProcessorCount;
     if (const char* z = getenv("ESFM_ORB_Z")) ctx->orb_z = atoi(z) != 0;
     if (const char* z = getenv("ESFM_TWO_PHASE")) ctx->two_phase = atoi(z) != 0;
+    if (const char* z = getenv("ESFM_TC16_EXACT")) ctx->tc16_exact = atoi(z) != 0;
     if (const char* eng = getenv("ESFM_HAMMING_ENGINE")) {
         if (!strcmp(eng, "tc") || !strcmp(eng, "tensor")) ctx->hamming_engine = ESFM_HAMMING_ENGINE_TC;
         else if (!strcmp(eng, "tc16")) ctx->hamming_engine = ESFM_HAMMING_ENGINE_TC16;
@@ -294,7 +295,7 @@ extern "C" int esfm_init(int device, void* cuda_stream, esfm_ctx_t** out) {
             e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
             if (e != cudaSuccess) return bail(ESFM_ERR_CUDA, "cudaEventCreate", e);
         }
-        e = cudaMalloc((void**)&cb.d_cursor, 2 * sizeof(unsigned long long));
+        e = cudaMalloc((void**)&cb.d_cursor, 3 * sizeof(unsigned long long));
         if (e != cudaSuccess) return bail(ESFM_ERR_NOMEM, "cudaMalloc", e);
     }
     {   // banks come and go (one per all-pairs call in the per-call API): they are allocated stream-ordered from a memory pool
@@ -816,7 +817,7 @@ int ensure_scratch(esfm_ctx* ctx, const esfm_bank* b, const ChunkPlan& pl, int n
             cb.pairs_cap = pl.chunk_pairs;
         }
         if (int rc = grow_pinned(&cb.h_pairs, &cb.h_pairs_cap, pl.chunk_pairs)) return rc;
-        const size_t meta = pl.chunk_pairs * (sizeof(int32_t) + sizeof(unsigned long long)) + 2 * sizeof(unsigned long long);
+        const size_t meta = pl.chunk_pairs * (sizeof(int32_t) + sizeof(unsigned long long)) + 3 * sizeof(unsigned long long);
         if (int rc = grow_pinned(&cb.h_meta, &cb.h_meta_bytes, meta)) return rc;
     }
     return ESFM_OK;
@@ -844,11 +845,16 @@ int ensure_kmajor_layout(esfm_ctx* ctx, esfm_bank* b) {
 
 // Tensor-core engines: the operand images of tc_layout.cuh.  z_mode: F32X64: 0 = 3xTF32 hi/lo images, 2 = the 16-bit split ("H")
 // images of sweep_win.cu; B256: 0 = +-1 FP8 images (also what sweep_win.cu reads), 1 = "Z" encoding.
+// The H images are followed by what win_fast_eps needs: float row_eps[total rows], frame_norm[n_frames].
+float* tch_row_eps(const esfm_bank* b) { return reinterpret_cast<float*>(b->d_tc + ((size_t)b->tile_off[b->n_frames] + 1) * kTchTileBytes); }
+float* tch_frame_norm(const esfm_bank* b) { return tch_row_eps(b) + b->row_off[b->n_frames]; }
+
 int ensure_tc_layout(esfm_ctx* ctx, esfm_bank* b, int z_mode) {
     if (b->tc_built && b->tc_z == z_mode) return ESFM_OK;
     b->tc_z = z_mode;
     const int n_tiles = b->tile_off[b->n_frames];
     b->tc_bytes = ((size_t)n_tiles + 1) * (b->kind == ESFM_KIND_F32X64 && z_mode != 2 ? (size_t)kTcTileBytes : (size_t)kTc8TileBytes);
+    if (b->kind == ESFM_KIND_F32X64 && z_mode == 2) b->tc_bytes += ((size_t)b->row_off[b->n_frames] + b->n_frames) * sizeof(float);
     if (!b->d_tc || b->tc_cap < b->tc_bytes) {
         if (b->d_tc) cudaFreeAsync(b->d_tc, ctx->stream);   // (stream-ordered: earlier sweeps have been enqueued before)
         b->d_tc = nullptr;
@@ -857,7 +863,8 @@ int ensure_tc_layout(esfm_ctx* ctx, esfm_bank* b, int z_mode) {
         b->tc_cap = b->tc_bytes;
     }
     cudaError_t e = b->kind == ESFM_KIND_F32X64
-            ? (z_mode == 2 ? launch_pack_tch((const float*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc, ctx->stream)
+            ? (z_mode == 2 ? launch_pack_tch((const float*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc,
+                                             tch_row_eps(b), tch_frame_norm(b), ctx->stream)
                            : launch_pack_tc((const float*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc, ctx->stream))
             : launch_pack_tc8((const uint32_t*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc, z_mode, ctx->stream);
     if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "tensor-core pack kernel launch failed: %s", cudaGetErrorString(e));
@@ -878,7 +885,7 @@ int units_per_pair(const esfm_ctx* ctx, const esfm_bank* b, size_t n_chunk_pairs
 int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, size_t n, double ratio, int cross_check, int32_t* knn_idx,
               float* knn_dist) {
     CUDA_TRY(cudaMemsetAsync(ctx->keys, 0xFF, n * 4 * (size_t)pl.stride * sizeof(u64), ctx->stream));
-    CUDA_TRY(cudaMemsetAsync(cb.d_cursor, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(cb.d_cursor, 0, 3 * sizeof(unsigned long long), ctx->stream));
     const bool tc = use_tc(ctx, b);
     // ORB "Z" encoding: the column index rides in the key, so every frame must have at most 2^15 rows; else the +-1 encoding
     // tc16 sweeps (sweep_win.cu) are ROWS-ONLY.  Their cross-check runs in TWO PHASES: (1) the rows-only sweep + ratio test, survivors claim
@@ -890,6 +897,8 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, si
     const bool two_phase = win_engine && cross_check && !knn_idx && ctx->two_phase;
     const bool win = win_engine && !knn_idx && (two_phase || !cross_check);
     const int zmode = (tc && !win && b->kind == ESFM_KIND_B256 && ctx->orb_z && b->max_rows <= kTcZMaxRows) ? 1 : 0;
+    // SURF: the rows-only sweep runs in fast mode (9 MMA slots per tile); the rows its error bound leaves unsettled are re-swept exactly
+    const bool win_fast = win && b->kind == ESFM_KIND_F32X64 && !ctx->tc16_exact;
     if (tc) { if (int rc = ensure_tc_layout(ctx, b, win && b->kind == ESFM_KIND_F32X64 ? 2 : zmode)) return rc; }
     else if (b->kind == ESFM_KIND_F32X64) { if (int rc = ensure_kmajor_layout(ctx, b)) return rc; }
     if ((b->kind == ESFM_KIND_F32X64 || tc) && !two_phase)
@@ -918,13 +927,13 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, si
     if (const char* dbg = getenv("ESFM_TC_DEBUG")) sp.debug_flags = atoi(dbg);
     sp.tc_qtiles = 1;
     sp.tc_kind = zmode ? kTcKindB256Z : b->kind;
+    sp.win_fast = win_fast ? 1 : 0;
     if (ctx->profiling) CUDA_TRY(cudaEventRecord(cb.ev_t0, ctx->stream));
     cudaError_t e = win ? launch_sweep_win(sp, ctx->sm_count, ctx->stream)
                   : tc ? launch_sweep_l2_tc(sp, ctx->sm_count, ctx->stream)
                        : (b->kind == ESFM_KIND_F32X64 ? launch_sweep_l2(sp, ctx->sm_count, ctx->stream)
                                                       : launch_sweep_hamming(sp, ctx->sm_count, ctx->stream));
     if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "sweep kernel launch failed: %s", cudaGetErrorString(e));
-    if (ctx->profiling) CUDA_TRY(cudaEventRecord(cb.ev_t1, ctx->stream));
     FinalizeParams fp{};
     fp.kind = b->kind;
     fp.rows_f32 = (const float*)b->d_rows;
@@ -950,6 +959,23 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, si
     fp.pair_cnt = cb.d_pair_cnt;
     fp.knn_idx = knn_idx;
     fp.knn_dist = knn_dist;
+    if (win_fast) {
+        // rows the fast sweep cannot settle -> the pair's gather list -> one exact sweep of just those rows (sweep time)
+        fp.row_eps = tch_row_eps(b);
+        fp.frame_norm = tch_frame_norm(b);
+        fp.fallback_rows = cb.d_cursor + 2;
+        e = launch_win_classify(fp, ctx->stream);
+        if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "fast-sweep classification kernel launch failed: %s", cudaGetErrorString(e));
+        SweepParams xp = sp;
+        xp.win_fast = 0;
+        xp.gather = fp.gather;
+        xp.gather_cnt = fp.gather_cnt;
+        xp.fallback = 1;
+        e = launch_sweep_win(xp, ctx->sm_count, ctx->stream);
+        if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "fallback sweep launch failed: %s", cudaGetErrorString(e));
+        ctx->stats.kernel_launches += 2;
+    }
+    if (ctx->profiling) CUDA_TRY(cudaEventRecord(cb.ev_t1, ctx->stream));
     e = launch_finalize(fp, ctx->stream);
     if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "finalize kernel launch failed: %s", cudaGetErrorString(e));
     cb.two_phase = two_phase;
@@ -957,6 +983,7 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, si
         SweepParams vp = sp;
         vp.gather = fp.gather;
         vp.gather_cnt = fp.gather_cnt;
+        vp.win_fast = 0;
         if (ctx->profiling) CUDA_TRY(cudaEventRecord(cb.ev_v0, ctx->stream));
         e = launch_sweep_win(vp, ctx->sm_count, ctx->stream);
         if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "verification sweep launch failed: %s", cudaGetErrorString(e));
@@ -1086,13 +1113,13 @@ int esfm::match_pairs_impl(esfm_bank* b, const esfm_pair_t* pairs, int64_t n_pai
         ChunkBuf& cb = ctx->buf[k & 1];
         CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, cb.ev_t2, 0));
         unsigned long long* h_cur = (unsigned long long*)cb.h_meta;
-        unsigned long long* h_off = h_cur + 2;
+        unsigned long long* h_off = h_cur + 3;
         int32_t* h_cnt = (int32_t*)(h_off + ch.n);
-        CUDA_TRY(cudaMemcpyAsync(h_cur, cb.d_cursor, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->copy_stream));
+        CUDA_TRY(cudaMemcpyAsync(h_cur, cb.d_cursor, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->copy_stream));
         CUDA_TRY(cudaMemcpyAsync(h_off, cb.d_pair_off, ch.n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->copy_stream));
         CUDA_TRY(cudaMemcpyAsync(h_cnt, cb.d_pair_cnt, ch.n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->copy_stream));
         CUDA_TRY(cudaEventRecord(cb.ev_meta, ctx->copy_stream));
-        ctx->stats.d2h_bytes += ch.n * (sizeof(int32_t) + sizeof(unsigned long long)) + 2 * sizeof(unsigned long long);
+        ctx->stats.d2h_bytes += ch.n * (sizeof(int32_t) + sizeof(unsigned long long)) + 3 * sizeof(unsigned long long);
         return ESFM_OK;
     };
     auto finish = [&](size_t k) -> int {            // chunk k has been finalised: book its pairs, bring its matches to the host
@@ -1101,10 +1128,11 @@ int esfm::match_pairs_impl(esfm_bank* b, const esfm_pair_t* pairs, int64_t n_pai
         CUDA_TRY(cudaEventSynchronize(cb.ev_meta));
         if (int rc = collect_timing(ctx, cb)) return rc;
         const unsigned long long* h_cur = (const unsigned long long*)cb.h_meta;
-        const unsigned long long* h_off = h_cur + 2;
+        const unsigned long long* h_off = h_cur + 3;
         const int32_t* h_cnt = (const int32_t*)(h_off + ch.n);
         const unsigned long long n_matches = h_cur[0];
         if ((int)h_cur[1] != 0 || n_matches > cb.arena_cap) return fail(ESFM_ERR_CAPACITY, "match arena overflow (internal sizing error)");
+        ctx->stats.fallback_rows += h_cur[2];
         const int seg = (int)res->segments.size();
         for (size_t i = 0; i < ch.n; ++i) {
             res->counts[ch.c0 + ch.order[i]] = h_cnt[i];

@@ -70,6 +70,13 @@ struct SweepParams {
     // (value, slice) of every gathered row lands in the pair's 4th key array at [slot].  NULL = a normal sweep.
     const int* gather;
     const int* gather_cnt;
+    // SURF (sweep_win.cu): 1 = FAST mode, the query enters as a = fp16(x) only: 8 kind::f16 MMAs + the norm step = 9 slots per tile instead
+    // of 13, values within win_fast_eps of the exact ones.  0 = exact mode (13 slots).
+    int win_fast;
+    // with `gather`: 1 = FALLBACK sweep, the gathered rows are rows of the pair's QUERY frame (the ones the fast sweep could not settle),
+    // swept in exact mode against the pair's train frame; their (best, second) keys overwrite rk1 / rk2 at the original row, marked with
+    // kWinExactMark.  0 = the role-swapped verification sweep above.
+    int fallback;
     int debug_flags;            // TC sweep pipeline probes ($ESFM_TC_DEBUG; results are WRONG when set): 1 = epilogue only drains,
                                 // 2 = no MMAs issued, 4 = no train-tile loads, 8 = no column events, 16 = no row selection, 32 = column events without their atomics, 64 = column events found but not handled
 };
@@ -99,6 +106,11 @@ struct FinalizeParams {
                                 // 2 = verdicts of the verification sweep + compaction
     int* gather;                // [n_pairs][stride] phase 1 out / the verification sweep's input
     int* gather_cnt;            // [n_pairs]
+    // SURF rows from the FAST sweep (SweepParams::win_fast; NULL = every row was swept in exact mode): per bank row |x - fp16(x)|_2,
+    // per frame the largest |x|_2 (launch_pack_tch) -> win_fast_eps.  Rows whose key carries kWinExactMark were re-swept exactly.
+    const float* row_eps;
+    const float* frame_norm;
+    unsigned long long* fallback_rows;   // win_classify: += rows put on the fallback list
     // optional raw knn output for one pair (esfm_knn2_pair)
     int32_t* knn_idx;
     float* knn_dist;
@@ -112,19 +124,43 @@ cudaError_t launch_pack_tc8(const uint32_t* rows, const int* frame_rows, const i
 cudaError_t launch_pack_tc(const float* rows, const int* frame_rows, const int* frame_row_off, const int* frame_tile_off,
                            int n_frames, int n_tiles_total, unsigned char* tc_main, cudaStream_t s);
 cudaError_t launch_pack_tch(const float* rows, const int* frame_rows, const int* frame_row_off, const int* frame_tile_off,
-                            int n_frames, int n_tiles_total, unsigned char* tc_main, cudaStream_t s);
+                            int n_frames, int n_tiles_total, unsigned char* tc_main, float* row_eps, float* frame_norm, cudaStream_t s);
 cudaError_t launch_sweep_l2(const SweepParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_sweep_win(const SweepParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_sweep_l2_tc(const SweepParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_sweep_hamming(const SweepParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_finalize(const FinalizeParams& p, cudaStream_t s);
+cudaError_t launch_win_classify(const FinalizeParams& p, cudaStream_t s);
 size_t sweep_l2_smem_bytes(int stages);
 size_t sweep_hamming_smem_bytes(int col_cap);
 int sweep_l2_max_rows();       // largest frame (rows) the L2 sweep supports
 int sweep_hamming_max_rows();
 
+// Low-word bit of a slice key (sweep_win.cu) whose row was swept in exact mode by the fallback sweep (slice ids stay below 2^30).
+constexpr uint32_t kWinExactMark = 0x80000000u;
+
 // ---- device helpers ------------------------------------------------------------------------------
 #ifdef __CUDACC__
+// Bound on |v' - v| for every train row t of a frame, v' = what the FAST SURF sweep ranks by (a_q.(a_t + b_t) - 1/2|q|^2 - 1/2|t|^2 in
+// fp32 accumulation, a = fp16(x), b = fp16(x - a)), v = -1/2 |q - t|^2 exactly (DESIGN.md section 5.0, "the fast-mode bound"):
+//     v' - v = -(q - a_q).t - a_q.r_t + rounding,    r_t = t - a_t - b_t,   |r_t| <= 2^-22 |t| + 2^-22 (64 dims, fp16 subnormals)
+// e_q = |q - a_q|_2, n_q / n_t = the largest row norms of the query / train frame (all rounded up).  The last term covers the fp32 sums
+// of the two half norms (2 x 64 fused steps) and the 9 MMA accumulations (17 addends each, truncated, none above m).
+// (Written with the _rn intrinsics, which the compiler never contracts: win_classify_kernel and finalize must compute the same bits.)
+__device__ __forceinline__ float win_fast_eps(float e_q, float n_q, float n_t) {
+    const float m = __fadd_rn(__fmul_rn(0.5f, __fadd_rn(__fmul_rn(n_q, n_q), __fmul_rn(n_t, n_t))), __fmul_rn(n_q, n_t));
+    const float r = __fmul_rn(__fadd_rn(n_q, e_q), __fmul_rn(0x1p-22f, __fadd_rn(n_t, 1.f)));
+    return __fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(e_q, n_t), r), __fmul_rn(0x1p-15f, m)), 1.001f);
+}
+// Ratio test on the sweep's 1/2 d^2 values s1 <= s2 of a row whose every value is within e of the exact one (e = 0: an exact-mode
+// sweep, whose own ~4e-7 is what the 0.1 % + 4e-6 margins absorb): 0 = fails for certain, 1 = passes for certain (and for e > 0 no other
+// column can be the nearest: the best slice holds it), 2 = to be decided on exact distances.
+__device__ __forceinline__ int win_ratio_class(float s1, float s2, float e, float r2) {
+    if (__fsub_rn(s1, e) > __fadd_rn(__fmul_rn(__fmul_rn(r2, __fadd_rn(s2, e)), 1.001f), 4e-6f)) return 0;
+    if (__fadd_rn(s1, e) < __fsub_rn(__fmul_rn(__fmul_rn(r2, __fsub_rn(s2, e)), 0.999f), 4e-6f) && (e == 0.f || __fsub_rn(s2, s1) > 2.f * e)) return 1;
+    return 2;
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {

@@ -107,10 +107,10 @@ __device__ __forceinline__ RowResult eval_row(const FinalizeParams& p, const u64
 }
 
 // ---- slice keys (sweep_win.cu): a row key's low word names a slice of train columns instead of one column ----
-//     id = (first column / 8) << 2 | width code         0: 8 columns, 1: 32, 2: 64, 3: 128
+//     id = (first column / 8) << 2 | width code         0: 8 columns, 1: 32, 2: 64, 3: 128      (| kWinExactMark: see SweepParams::fallback)
 // The column itself is found HERE, by evaluating the slice exactly -- and only for rows that can still pass the ratio test.
 __device__ __forceinline__ void win_range(u64 key, int ft, int& c0, int& c1) {
-    const uint32_t id = (uint32_t)key;
+    const uint32_t id = (uint32_t)key & ~kWinExactMark;
     c0 = (int)(id >> 2) * 8;
     const uint32_t w = id & 3u;
     c1 = min(c0 + (w == 0u ? 8 : (w == 1u ? 32 : (w == 2u ? 64 : 128))), ft);
@@ -156,9 +156,10 @@ __device__ __forceinline__ void top2_merge(float& d1, int& i1, float& d2, int& i
 // evaluated are served four at a time by groups of eight lanes -- one candidate column per lane and step, all loads of a step in flight
 // together -- instead of every lane walking its own slice serially (a quarter of the lanes busy, eight dependent gathers each: that walk
 // was 90 % of the kernel's time).  Each distance is still computed by ONE lane with l2_direct (the oracle's summation order).
+// `e`: SURF, the row's values come from the fast sweep and are within e of the exact ones (0: exact mode).
 template <int KIND>
-__device__ __forceinline__ RowResult eval_rows_win(const FinalizeParams& p, u64 k1, u64 k2, const float* qrows, const float* trows, const uint4* qbits,
-                                                   const uint4* tbits, int q, int ft, bool valid) {
+__device__ __forceinline__ RowResult eval_rows_win(const FinalizeParams& p, u64 k1, u64 k2, float e, const float* qrows, const float* trows,
+                                                   const uint4* qbits, const uint4* tbits, int q, int ft, bool valid) {
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31, grp = lane >> 3, sub = lane & 7;
     const bool has1 = valid && k1 != kKeyInit, has2 = valid && k2 != kKeyInit;
@@ -177,18 +178,17 @@ __device__ __forceinline__ RowResult eval_rows_win(const FinalizeParams& p, u64 
         pass = has1 && (no_ratio || (has2 && (double)d1 < p.ratio * (double)d2));
         scan_a = pass;
     } else if (has1) {
-        // the sweep ranked 1/2 d^2 in expansion form (error ~4e-7 absolute): decide far-from-the-boundary rows on those values,
-        // evaluate the rest -- and every reported distance -- in direct form
+        // the sweep ranked 1/2 d^2 in expansion form (error ~4e-7 absolute, or e): decide far-from-the-boundary rows on those values,
+        // evaluate the rest -- and every reported distance -- in direct form.  (A fast-mode row never lands in between: win_classify
+        // has sent those to the fallback sweep.)
         const float s1 = __uint_as_float((uint32_t)(k1 >> 32)), s2 = has2 ? __uint_as_float((uint32_t)(k2 >> 32)) : inf;
         if (no_ratio) { pass = true; scan_a = true; }
         else if (has2 && p.ratio > 0.0) {
-            const float r2 = (float)(p.ratio * p.ratio);
-            const bool clear_fail = s1 > r2 * s2 * 1.001f + 4e-6f;
-            const bool clear_pass = s1 < r2 * s2 * 0.999f - 4e-6f;
-            if (!clear_fail) {
+            const int cls = win_ratio_class(s1, s2, e, (float)(p.ratio * p.ratio));
+            if (cls != 0) {
                 scan_a = true;
-                pass = clear_pass;
-                if (!clear_pass) { scan_b = true; exact_ratio = true; }
+                pass = cls == 1;
+                if (cls == 2) { scan_b = true; exact_ratio = true; }
             }
         }
         if (scan_b && a0 >= b0 && a1 <= b1) scan_a = false;       // slice a lies inside slice b: one evaluation
@@ -370,12 +370,16 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
         __syncthreads();
     }
     if (p.win_keys) {
+        const bool fast = KIND == ESFM_KIND_F32X64 && p.row_eps;
+        const float* row_eps = fast ? p.row_eps + p.frame_row_off[pd.q_frame] : nullptr;
+        const float nq = fast ? p.frame_norm[pd.q_frame] : 0.f, nt = fast ? p.frame_norm[pd.t_frame] : 0.f;
         // slice keys: every warp takes 32 consecutive rows per iteration and evaluates their slices cooperatively
         for (int q0 = warp * 32; q0 < fq; q0 += kFinThreads) {
             const int q = q0 + lane;
             const bool valid = q < fq;
             const u64 k1 = valid ? rk1[q] : kKeyInit, k2 = valid ? rk2[q] : kKeyInit;
-            const RowResult r = eval_rows_win<KIND>(p, k1, k2, qrows, trows, qbits, tbits, q, ft, valid);
+            const float e = (fast && !((uint32_t)k1 & kWinExactMark)) ? win_fast_eps(row_eps[q], nq, nt) : 0.f;
+            const RowResult r = eval_rows_win<KIND>(p, k1, k2, e, qrows, trows, qbits, tbits, q, ft, valid);
             if (!valid) continue;
             rk1[q] = r.keep ? make_key(__float_as_uint(r.d1), (uint32_t)r.t1) : kKeyInit;
             mine += r.keep ? 1u : 0u;
@@ -383,9 +387,10 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
                 // Who could beat a survivor (q, t) at its own train row t?  A row whose NEAREST train row is t (another survivor: settled by
                 // the claims below; a row that failed the ratio test: counted in histogram A by its best value), or a row for which t is at
                 // best second (then its second-best value is <= its distance to t: histogram B, every row).  A survivor whose distance
-                // lies below every such value needs no verification sweep.
-                if (k2 != kKeyInit) atomicAdd(&s_hist[1][fin_bucket<KIND>(__uint_as_float((uint32_t)(k2 >> 32)))], 1u);
-                if (!r.keep && k1 != kKeyInit) atomicAdd(&s_hist[0][fin_bucket<KIND>(__uint_as_float((uint32_t)(k1 >> 32)))], 1u);
+                // lies below every such value needs no verification sweep.  Fast-mode values enter as lower bounds, value - e: the k-th
+                // smallest of a row's values moves by at most e, whichever column the sweep named.
+                if (k2 != kKeyInit) atomicAdd(&s_hist[1][fin_bucket<KIND>(__uint_as_float((uint32_t)(k2 >> 32)) - e)], 1u);
+                if (!r.keep && k1 != kKeyInit) atomicAdd(&s_hist[0][fin_bucket<KIND>(__uint_as_float((uint32_t)(k1 >> 32)) - e)], 1u);
                 // every train row some survivor points at is claimed by the nearest such query row (lowest index on ties)
                 if (r.keep) atomicMin(const_cast<u64*>(ck1) + r.t1, make_key(__float_as_uint(r.d1), (uint32_t)q));
             }
@@ -492,7 +497,47 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
     }
 }
 
+// SURF fast sweep -> which rows need the exact fallback sweep, from the sweep's values alone (no descriptor reads): every row that
+// eval_rows_win could not decide on its values (win_ratio_class == 2), and with ratio = inf every row whose nearest column is not
+// certain (s2 - s1 <= 2 e).  Their indices go on the pair's gather list, any order (the fallback sweep writes back by row index).
+__global__ void __launch_bounds__(kFinThreads) win_classify_kernel(const FinalizeParams p) {
+    const int pair = blockIdx.x;
+    const PairDesc pd = p.pairs[pair];
+    const int fq = p.frame_rows[pd.q_frame], ft = p.frame_rows[pd.t_frame];
+    const bool no_ratio = p.ratio == __longlong_as_double(0x7ff0000000000000LL);
+    __shared__ unsigned int s_cnt;
+    if (threadIdx.x == 0) s_cnt = 0;
+    __syncthreads();
+    if (fq > 0 && ft >= (no_ratio ? 1 : 2) && (no_ratio || p.ratio > 0.0)) {      // (else finalize emits nothing for the pair)
+        const u64* rk1 = p.keys + (size_t)pair * 4 * p.stride;
+        const u64* rk2 = rk1 + p.stride;
+        const float* row_eps = p.row_eps + p.frame_row_off[pd.q_frame];
+        const float nq = p.frame_norm[pd.q_frame], nt = p.frame_norm[pd.t_frame];
+        const float r2 = (float)(p.ratio * p.ratio);
+        int* gl = p.gather + (size_t)pair * p.stride;
+        for (int q = threadIdx.x; q < fq; q += kFinThreads) {
+            const u64 k1 = rk1[q], k2 = rk2[q];
+            if (k1 == kKeyInit || k2 == kKeyInit) continue;          // no second column: nothing to rank
+            const float s1 = __uint_as_float((uint32_t)(k1 >> 32)), s2 = __uint_as_float((uint32_t)(k2 >> 32));
+            const float e = win_fast_eps(row_eps[q], nq, nt);
+            const bool unsettled = no_ratio ? !(s2 - s1 > 2.f * e) : win_ratio_class(s1, s2, e, r2) == 2;
+            if (unsettled) gl[atomicAdd(&s_cnt, 1u)] = q;
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        p.gather_cnt[pair] = (int)s_cnt;
+        if (s_cnt) atomicAdd(p.fallback_rows, (unsigned long long)s_cnt);
+    }
+}
+
 }  // namespace
+
+cudaError_t launch_win_classify(const FinalizeParams& p, cudaStream_t s) {
+    if (p.n_pairs <= 0) return cudaSuccess;
+    win_classify_kernel<<<p.n_pairs, kFinThreads, 0, s>>>(p);
+    return cudaGetLastError();
+}
 
 cudaError_t launch_finalize(const FinalizeParams& p, cudaStream_t s) {
     if (p.n_pairs <= 0) return cudaSuccess;

@@ -54,7 +54,7 @@ struct ChunkBuf {
     unsigned long long* d_pair_off = nullptr;
     int32_t* d_pair_cnt = nullptr;
     size_t pairs_cap = 0;
-    unsigned long long* d_cursor = nullptr;      // [0] arena cursor, [1] overflow flag
+    unsigned long long* d_cursor = nullptr;      // [0] arena cursor, [1] overflow flag, [2] rows re-swept by the SURF fallback sweep
     esfm_dmatch_t* arena = nullptr;              // dense match arena of the chunk
     size_t arena_cap = 0;                        // in matches
     uint64_t generation = 0;                     // bumped whenever the arena is overwritten
@@ -91,6 +91,8 @@ struct esfm_ctx {
     int* gather_cnt = nullptr;     size_t gather_cnt_elems = 0;     // two-phase cross-check: train rows to verify, per pair of the chunk
     int two_phase = 1;                     // cross-check of the tc16 sweeps as ratio test -> verification sweep over the surviving train rows
                                            // ($ESFM_TWO_PHASE=0: column minima inside the one sweep, as the other engines do)
+    int tc16_exact = 0;                    // $ESFM_TC16_EXACT=1: SURF tc16 sweeps in exact mode (13 MMA slots per tile) instead of fast mode
+                                           // (9 slots) + exact fallback sweep of the rows it cannot settle
     esfm::ChunkBuf buf[2];
     // a pool of large pinned buffers that banks (upload staging) and results (downloaded matches) borrow, so steady-state
     // calls never allocate or zero-fill host memory

@@ -11,7 +11,9 @@
 // only does for the rows that can pass the ratio test.  The epilogue therefore needs VALUES only:
 //   * SURF (KIND = ESFM_KIND_F32X64, "H" split of tc_layout.cuh): 12 x tcgen05.mma.kind::f16 (a = fp16(x), b = fp16(x - a);
 //     b_q.a_t + a_q.b_t + a_q.a_t, fp32 accumulation; fp16 subnormals are honoured by the tensor core: h16_probe.cu) + the exact
-//     kind::tf32 half-norm step = 13 MMA slots per 128 x 128 tile instead of 25, tile image 36 KB instead of 68 KB.  Epilogue:
+//     kind::tf32 half-norm step = 13 MMA slots per 128 x 128 tile instead of 25, tile image 36 KB instead of 68 KB.  FAST mode
+//     (SweepParams::win_fast, the rows-only sweep's default) drops b_q: 8 + 1 = 9 slots, values within win_fast_eps (esfm_internal.cuh);
+//     the rows that bound cannot settle are swept again in exact mode (SweepParams::fallback, finalize.cu win_classify_kernel).  Epilogue:
 //     a branch-free tournament over the 32 accumulators of a pass gives the pass's two largest -1/2 d^2, eleven selects merge them
 //     into the running (k1, w1, k2, w2).
 //   * ORB (KIND = ESFM_KIND_B256): the +-1 FP8 operands of sweep_l2_tc.cu with FP16 ACCUMULATORS (-2 hamming, exact; pad rows
@@ -94,7 +96,8 @@ __device__ __forceinline__ void win_merge(float p1, int id1, float p2, int id2, 
 }
 
 // work decoding: a normal sweep takes (query frame, train frame) from the pair list; the verification sweep of the two-phase
-// cross-check swaps the roles and reads its query rows through the pair's gather list
+// cross-check swaps the roles and reads its query rows through the pair's gather list; the fallback sweep reads them through the list
+// without swapping
 struct WinUnit {
     int pair, q_frame, t_frame;
     int fq;              // query rows of this unit's pair (gathered rows in a verification sweep)
@@ -108,8 +111,8 @@ __device__ __forceinline__ WinUnit win_decode_unit(const SweepParams& p, int uni
     const PairDesc pd = p.pairs[u.pair];
     int nqt;
     if (p.gather) {
-        u.q_frame = pd.t_frame;
-        u.t_frame = pd.q_frame;
+        u.q_frame = p.fallback ? pd.q_frame : pd.t_frame;
+        u.t_frame = p.fallback ? pd.t_frame : pd.q_frame;
         u.fq = p.gather_cnt[u.pair];
         nqt = (u.fq + kTile - 1) / kTile;
     } else {
@@ -227,11 +230,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_win_kernel(const SweepPar
                             for (int ks = 0; ks < 8; ++ks)
                                 tc_mma_f8_ts(d, acol + ks * 8, td + (uint64_t)(((ks >> 2) * 1024 + (ks & 3) * 32) >> 4), id_main, ks > 0);
                         } else {
-                            // small terms first: b_q.a_t, a_q.b_t, then a_q.a_t; a k-step = 16 halves = 32 bytes of the 128-byte row
+                            // small terms first: b_q.a_t (exact mode only), a_q.b_t, then a_q.a_t; a k-step = 16 halves = 32 bytes of the
+                            // 128-byte row
+                            if (!p.win_fast) {
 #pragma unroll
-                            for (int ks = 0; ks < 4; ++ks) tc_mma_f16_ts(d, acol + 32 + ks * 8, td + (uint64_t)((ks * 32) >> 4), id_main, ks > 0);
+                                for (int ks = 0; ks < 4; ++ks) tc_mma_f16_ts(d, acol + 32 + ks * 8, td + (uint64_t)((ks * 32) >> 4), id_main, ks > 0);
+                            }
 #pragma unroll
-                            for (int ks = 0; ks < 4; ++ks) tc_mma_f16_ts(d, acol + ks * 8, td + (uint64_t)((1024 + ks * 32) >> 4), id_main, true);
+                            for (int ks = 0; ks < 4; ++ks)
+                                tc_mma_f16_ts(d, acol + ks * 8, td + (uint64_t)((1024 + ks * 32) >> 4), id_main, ks > 0 || !p.win_fast);
 #pragma unroll
                             for (int ks = 0; ks < 4; ++ks) tc_mma_f16_ts(d, acol + ks * 8, td + (uint64_t)((ks * 32) >> 4), id_main, true);
                             tc_mma_tf32(d, qad, tad, tc_idesc_tf32(128, 128), true);   // - 1/2|q|^2 - 1/2|t|^2, exact
@@ -302,7 +309,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_win_kernel(const SweepPar
                     *reinterpret_cast<float4*>(qa) = make_float4(1.f, 1.f, 1.f, hqh);
                     *reinterpret_cast<float4*>(qa + 128) = make_float4(hqm, hql, 0.f, 0.f);
                     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    // pass 2: the row again (L1/L2 hit), 16 dims at a time -> 8 columns of a (fp16 pairs) and 8 of b
+                    // pass 2: the row again (L1/L2 hit), 16 dims at a time -> 8 columns of a (fp16 pairs) and, in exact mode, 8 of b
 #pragma unroll 1
                     for (int m = 0; m < 4; ++m) {
                         uint32_t ca[8], cb[8];
@@ -311,13 +318,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_win_kernel(const SweepPar
                             float4 x = __ldg(xr + 4 * m + h);
                             if (!valid) x = make_float4(0.f, 0.f, 0.f, 0.f);
                             const __half2 a0 = __floats2half2_rn(x.x, x.y), a1 = __floats2half2_rn(x.z, x.w);
-                            const float2 f0 = __half22float2(a0), f1 = __half22float2(a1);
-                            const __half2 b0 = __floats2half2_rn(x.x - f0.x, x.y - f0.y), b1 = __floats2half2_rn(x.z - f1.x, x.w - f1.y);
                             ca[2 * h] = *reinterpret_cast<const uint32_t*>(&a0); ca[2 * h + 1] = *reinterpret_cast<const uint32_t*>(&a1);
-                            cb[2 * h] = *reinterpret_cast<const uint32_t*>(&b0); cb[2 * h + 1] = *reinterpret_cast<const uint32_t*>(&b1);
+                            if (!p.win_fast) {
+                                const float2 f0 = __half22float2(a0), f1 = __half22float2(a1);
+                                const __half2 b0 = __floats2half2_rn(x.x - f0.x, x.y - f0.y), b1 = __floats2half2_rn(x.z - f1.x, x.w - f1.y);
+                                cb[2 * h] = *reinterpret_cast<const uint32_t*>(&b0); cb[2 * h + 1] = *reinterpret_cast<const uint32_t*>(&b1);
+                            }
                         }
                         tmem_st8(acol + m * 8, ca);
-                        tmem_st8(acol + 32 + m * 8, cb);
+                        if (!p.win_fast) tmem_st8(acol + 32 + m * 8, cb);
                     }
                 }
                 tmem_st_wait();
@@ -457,7 +466,14 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_win_kernel(const SweepPar
                 }
                 asm volatile("bar.sync 1, %0;" ::"n"(kTcEpiThreads) : "memory");
                 if (group == 0) {
-                    if (p.gather) {
+                    if (p.gather && p.fallback) {
+                        // fallback sweep: gathered row `qrow` is row gl[qrow] of the query frame (kKeyInit keeps its value under the mark)
+                        if ((int)qrow < u.fq) {
+                            const int r = __ldg(p.gather + (size_t)u.pair * p.stride + qrow);
+                            rk1[r] = mkey[trow] | kWinExactMark;
+                            rk2[r] = mkey[kTile + trow] | kWinExactMark;
+                        }
+                    } else if (p.gather) {
                         rk1[3 * (size_t)p.stride + qrow] = mkey[trow];      // verification sweep: the best (value, slice) of gathered row `qrow`
                     } else {
                         rk1[qrow] = mkey[trow];

@@ -81,10 +81,11 @@ typedef struct esfm_stats_t {
     uint64_t d2h_bytes;        /* device->host bytes copied */
     uint64_t comparisons;      /* descriptor comparisons evaluated (rows_q * rows_t per pair, counted once) */
     uint64_t pairs;            /* image pairs matched */
-    double last_sweep_ms;      /* device time of the most recent distance/top-2 sweep kernel (CUDA events) */
+    double last_sweep_ms;      /* device time of the most recent distance/top-2 sweep kernel (CUDA events; SURF tc16: with the fallback sweep) */
     double last_finalize_ms;   /* device time of the most recent refine/ratio/cross-check/compaction kernel */
     double sweep_ms_total;     /* sum of sweep kernel device times */
     uint64_t sweep_launches;   /* number of sweep kernel launches */
+    uint64_t fallback_rows;    /* SURF tc16: query rows the 9-slot sweep could not settle, re-swept in exact (13-slot) mode */
 } esfm_stats_t;
 
 int esfm_abi_version(void);
