@@ -335,15 +335,16 @@ class Context:
                                              ctypes.byref(prm), mask.ctypes.data, out.ctypes.data))
         return mask[:total], out[:n_pairs]
 
-    def two_view_depth(self, pts1, pts2, K, R, t, random_rate=20) -> float:
-        """esfm_two_view_depth: MotionEstimator::getDepthFast for one pair (every random_rate-th match, [I|0] and [R|t])."""
+    def two_view_depth(self, pts1, pts2, K, R, t, random_rate=20, return_used=False):
+        """esfm_two_view_depth: MotionEstimator::getDepthFast for one pair (every random_rate-th match, [I|0] and [R|t]).  Returns the mean
+        depth, or (mean depth, number of matches triangulated) with return_used=True."""
         pts1 = np.ascontiguousarray(pts1, np.float32).reshape(-1, 2)
         pts2 = np.ascontiguousarray(pts2, np.float32).reshape(-1, 2)
         K, R, t = (np.ascontiguousarray(a, np.float64) for a in (K, R, t))
         depth, used = c_double(0.0), c_int32(0)
         _check(self._lib.esfm_two_view_depth(self._h, len(pts1), pts1.ctypes.data, pts2.ctypes.data, K.ctypes.data, R.ctypes.data, t.ctypes.data,
                                              int(random_rate), ctypes.byref(depth), ctypes.byref(used)))
-        return depth.value
+        return (depth.value, used.value) if return_used else depth.value
 
     def orb_extract(self, image, max_features: int = 5000, want_descriptors: bool = True):
         """esfm_orb_extract: FeatureMatching::detectFeaturesORB (feature_matching.cpp:14-41) for one image -- uint8 [rows, cols] (gray) or

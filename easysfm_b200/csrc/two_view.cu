@@ -248,15 +248,18 @@ __global__ void __launch_bounds__(kTvPoseThreads) tv_pose_kernel(const double2* 
 }
 
 // getDepthFast on its own (estimate_motion.cpp:234-283): every random_rate-th of the GIVEN matches triangulated with [I|0], [R|t]; mean norm.
-// One block; deterministic summation (per-thread partial sums added in thread order).
-__global__ void __launch_bounds__(kTvPoseThreads) tv_depth_kernel(const float* __restrict__ p1, const float* __restrict__ p2, int n, const double* __restrict__ K,
-                                                                   const double* __restrict__ Rt, int random_rate, double* __restrict__ out) {
+// One block; deterministic summation (per-thread partial sums added in thread order).  Index, stride and n are 64-bit: random_rate may be
+// anything up to INT_MAX, and threadIdx.x * random_rate or 128 * random_rate would wrap in 32 bits.
+__global__ void __launch_bounds__(kTvPoseThreads) tv_depth_kernel(const float* __restrict__ p1, const float* __restrict__ p2, long long n,
+                                                                   const double* __restrict__ K, const double* __restrict__ Rt, int random_rate,
+                                                                   double* __restrict__ out) {
     __shared__ double sh_d[kTvPoseThreads];
-    __shared__ int sh_n[kTvPoseThreads];
+    __shared__ long long sh_n[kTvPoseThreads];
     const double fx = K[0], fy = K[4], cx = K[2], cy = K[5];
     double acc = 0.0;
-    int used = 0;
-    for (int i = threadIdx.x * random_rate; i < n; i += kTvPoseThreads * random_rate) {
+    long long used = 0;
+    const long long stride = (long long)kTvPoseThreads * random_rate;
+    for (long long i = (long long)threadIdx.x * random_rate; i < n; i += stride) {
         double Q[4];
         tv::triangulate_dlt(Rt, Rt + 9, ((double)p1[2 * i] - cx) / fx, ((double)p1[2 * i + 1] - cy) / fy, ((double)p2[2 * i] - cx) / fx,
                             ((double)p2[2 * i + 1] - cy) / fy, Q);
@@ -269,7 +272,7 @@ __global__ void __launch_bounds__(kTvPoseThreads) tv_depth_kernel(const float* _
     __syncthreads();
     if (threadIdx.x == 0) {
         double sum = 0.0;
-        int cnt = 0;
+        long long cnt = 0;
         for (int w = 0; w < kTvPoseThreads; ++w) { sum += sh_d[w]; cnt += sh_n[w]; }
         out[0] = cnt > 0 ? sum / cnt : 0.0;
         out[1] = (double)cnt;
@@ -388,7 +391,7 @@ extern "C" int esfm_two_view_depth(esfm_ctx_t* ctx, int64_t n_matches, const flo
     CUDA_TRY(cudaMemcpyAsync(d_p1.p, pts1, (size_t)n_matches * 8, cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(d_p2.p, pts2, (size_t)n_matches * 8, cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(d_par.p, par, sizeof par, cudaMemcpyHostToDevice, s));
-    tv_depth_kernel<<<1, kTvPoseThreads, 0, s>>>(d_p1.as<float>(), d_p2.as<float>(), (int)n_matches, d_par.as<double>(), d_par.as<double>() + 9, random_rate,
+    tv_depth_kernel<<<1, kTvPoseThreads, 0, s>>>(d_p1.as<float>(), d_p2.as<float>(), (long long)n_matches, d_par.as<double>(), d_par.as<double>() + 9, random_rate,
                                                  d_out.as<double>());
     CUDA_TRY(cudaGetLastError());
     double out[2];

@@ -194,8 +194,9 @@ def decompose_essential(E):
     return U @ W @ Vt, U @ W.T @ Vt, U[:, 2].copy()
 
 
-def recover_pose(E, pts1, pts2, K, mask, dist=50.0):
-    """cv::recoverPose(E, pts1, pts2, K, R, t, mask) (calib3d five-point.cpp): returns (R, t, n_good, mask_out)."""
+def cheirality_counts(E, pts1, pts2, K, mask, dist=50.0):
+    """recoverPose's four candidates (R1, t), (R2, t), (R1, -t), (R2, -t) and, for each, the masked matches triangulated in front of both
+    cameras and nearer than `dist`: returns (candidates, counts, per-match uint8 masks)."""
     K = np.asarray(K, np.float64)
     n1, n2 = normalise(pts1, K), normalise(pts2, K)
     R1, R2, t = decompose_essential(E)
@@ -212,7 +213,13 @@ def recover_pose(E, pts1, pts2, K, mask, dist=50.0):
         ok &= (X2[:, 2] > 0) & (X2[:, 2] < dist)
         ok &= mask.astype(bool)
         goods.append(int(ok.sum()))
-        masks.append(ok)
+        masks.append(ok.astype(np.uint8))
+    return cands, goods, masks
+
+
+def recover_pose(E, pts1, pts2, K, mask, dist=50.0):
+    """cv::recoverPose(E, pts1, pts2, K, R, t, mask) (calib3d five-point.cpp): returns (R, t, n_good, mask_out)."""
+    cands, goods, masks = cheirality_counts(E, pts1, pts2, K, mask, dist)
     g1, g2, g3, g4 = goods
     if g1 >= g2 and g1 >= g3 and g1 >= g4:
         k = 0
@@ -222,7 +229,7 @@ def recover_pose(E, pts1, pts2, K, mask, dist=50.0):
         k = 2
     else:
         k = 3
-    return cands[k][0], cands[k][1], goods[k], masks[k].astype(np.uint8)
+    return cands[k][0], cands[k][1], goods[k], masks[k]
 
 
 def mean_depth(R, t, pts1, pts2, K, mask, random_rate=1):
@@ -238,12 +245,12 @@ def mean_depth(R, t, pts1, pts2, K, mask, random_rate=1):
     return float(np.linalg.norm(X, axis=1).mean())
 
 
-def estimate_two_view(pts1, pts2, K, prob=0.99, thre=1.0, max_iters=1000, seed=0, pair=0, random_rate=1):
-    """The whole of estimate2D2D_E5P_RANSAC + getDepthFast for one image pair.  Returns a dict."""
+def estimate_two_view(pts1, pts2, K, prob=0.99, thre=1.0, max_iters=1000, seed=0, pair=0, random_rate=1, dist=50.0):
+    """The whole of estimate2D2D_E5P_RANSAC + getDepthFast for one image pair; `dist` is recoverPose's distance threshold.  Returns a dict."""
     E, mask, iters = find_essential_ransac(pts1, pts2, K, prob, thre, max_iters, seed, pair)
     out = {"E": E, "mask": mask, "iters": iters, "n_inliers": int(mask.sum()), "R": None, "t": None, "n_good": 0, "depth": float("nan")}
     if E is None:
         return out
-    R, t, good, pmask = recover_pose(E, pts1, pts2, K, mask)
+    R, t, good, pmask = recover_pose(E, pts1, pts2, K, mask, dist)
     out.update(R=R, t=t, n_good=good, depth=mean_depth(R, t, pts1, pts2, K, mask, random_rate))
     return out

@@ -12,7 +12,7 @@ import pytest
 
 from oracle import two_view_oracle as tvo
 from golden_util import load
-from two_view_util import dir_angle_deg, dptr, host_lib, rot_angle_deg, scene
+from two_view_util import DEGENERATE, degenerate_scene, dir_angle_deg, dptr, host_lib, project, random_K, rot_angle_deg, scene
 
 
 def _same_up_to_sign(E, F, tol):
@@ -88,6 +88,56 @@ def test_oracle_ransac_statistics_vs_cv2():
         assert dir_angle_deg(r["t"], t) <= max(6.0, 3.0 * dir_angle_deg(tcv, t))      # (raw RANSAC models, no refinement: degrees, not arc minutes)
         inl_true = np.arange(len(x1)) >= int(outl * len(x1))
         assert (r["mask"].astype(bool) & ~inl_true).sum() <= 0.05 * r["n_inliers"] + 3      # few gross outliers accepted
+
+
+def test_oracle_cheirality_distance_argument():
+    """estimate_two_view's `dist` reaches recoverPose: its pose, count and depth are recover_pose's with that threshold, and a threshold
+    inside the scene's depth range (4 .. 9) drops points that the default keeps."""
+    K, x1, x2, _, _ = scene(300, 0.3, 0.2, 61)
+    full = tvo.estimate_two_view(x1, x2, K, 0.99, 1.0, 1000, seed=2, pair=9, random_rate=3)
+    near = tvo.estimate_two_view(x1, x2, K, 0.99, 1.0, 1000, seed=2, pair=9, random_rate=3, dist=8.0)
+    for r, d in ((full, 50.0), (near, 8.0)):
+        R, t, good, _ = tvo.recover_pose(r["E"], x1, x2, K, r["mask"], d)
+        assert np.array_equal(r["R"], R) and np.array_equal(r["t"], t) and r["n_good"] == good
+        assert r["depth"] == tvo.mean_depth(R, t, x1, x2, K, r["mask"], 3)
+    assert np.array_equal(near["E"], full["E"]) and np.array_equal(near["mask"], full["mask"])
+    assert 0 < near["n_good"] < full["n_good"]
+
+
+@pytest.mark.parametrize("noise", [0.0, 0.3])
+def test_degenerate_generators(noise):
+    """Each degenerate scene is the geometry it claims: points on a plane or a line, t = 0, |t| = 1e-6, depth x 1e4, every correspondence
+    2 or 3 times, one correspondence n times, x1 == x2; without noise the pixels are the projections of X."""
+    for s, kind in enumerate(DEGENERATE):
+        K, x1, x2, R, t, X = degenerate_scene(kind, 200, noise, 70 + s, random_K(np.random.default_rng(s)))
+        assert x1.shape == x2.shape == (len(X), 2) and x1.dtype == np.float32
+        assert np.all(X[:, 2] > 0) and np.all((X @ R.T + t)[:, 2] > 0)
+        if noise == 0.0:
+            scale = max(1.0, np.abs(project(K, X)).max())
+            np.testing.assert_allclose(x1, project(K, X), atol=1e-6 * scale)
+            np.testing.assert_allclose(x2, project(K, X @ R.T + t), atol=1e-6 * scale)
+        sv = np.linalg.svd(X - X.mean(0), compute_uv=False)
+        if kind == "planar":
+            assert sv[2] <= 1e-12 * sv[0] and sv[1] > 0.1 * sv[0]
+            np.testing.assert_allclose(X[:, 2], 6.0 + 0.4 * X[:, 0] - 0.3 * X[:, 1], atol=1e-12)
+        if kind == "collinear":
+            assert sv[1] <= 1e-12 * sv[0]
+        if kind in ("rotation", "same"):
+            assert np.array_equal(t, np.zeros(3))
+        if kind == "baseline":
+            assert abs(np.linalg.norm(t) - 1e-6) <= 1e-18
+        if kind == "far":
+            assert X[:, 2].min() >= 4e4 and X[:, 2].max() <= 9e4 and abs(np.linalg.norm(t) - 1.0) < 1e-12
+        if kind == "repeated":
+            rows, inv, counts = np.unique(np.c_[x1, x2], axis=0, return_inverse=True, return_counts=True)
+            assert len(rows) == 200 and set(counts.tolist()) == {2, 3} and len(x1) == counts.sum()
+            assert not np.all(np.diff(inv.ravel()) >= 0)                        # shuffled, not in runs
+        if kind == "identical":
+            assert len(np.unique(np.c_[x1, x2], axis=0)) == 1 and len(x1) == 200
+        if kind == "same":
+            assert np.array_equal(x1, x2) and np.array_equal(R, np.eye(3))
+        if kind not in ("repeated", "identical"):
+            assert len(np.unique(np.c_[x1, x2], axis=0)) == len(x1)
 
 
 # --------------------------------------------------------------------------------------------------------------------------------------
