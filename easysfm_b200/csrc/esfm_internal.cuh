@@ -154,7 +154,9 @@ __device__ __forceinline__ float win_fast_eps(float e_q, float n_q, float n_t) {
 }
 // Ratio test on the sweep's 1/2 d^2 values s1 <= s2 of a row whose every value is within e of the exact one (e = 0: an exact-mode
 // sweep, whose own ~4e-7 is what the 0.1 % + 4e-6 margins absorb): 0 = fails for certain, 1 = passes for certain (and for e > 0 no other
-// column can be the nearest: the best slice holds it), 2 = to be decided on exact distances.
+// column can be the nearest: the best slice holds it), 2 = to be decided on exact distances.  SURF chain keys (sweep_win.cu): s2 is the best
+// value OUTSIDE the best chain, an upper bound on the true second (+inf: no second chain), so 0 stays certain and 1 speaks for the columns
+// outside the best chain only: finalize tests the best chain's own second exactly.
 __device__ __forceinline__ int win_ratio_class(float s1, float s2, float e, float r2) {
     if (__fsub_rn(s1, e) > __fadd_rn(__fmul_rn(__fmul_rn(r2, __fadd_rn(s2, e)), 1.001f), 4e-6f)) return 0;
     if (__fadd_rn(s1, e) < __fsub_rn(__fmul_rn(__fmul_rn(r2, __fsub_rn(s2, e)), 0.999f), 4e-6f) && (e == 0.f || __fsub_rn(s2, s1) > 2.f * e)) return 1;

@@ -30,6 +30,7 @@ template <int KIND> __device__ __forceinline__ int fin_bucket(float v) {
 struct RowResult {
     int t1;
     float d1;
+    float d2;       // SURF slice keys: the second of the columns finalize evaluated (+inf: none), a bound for histogram B
     bool keep;
 };
 
@@ -58,6 +59,7 @@ __device__ __forceinline__ RowResult eval_row(const FinalizeParams& p, const u64
     r.keep = false;
     r.t1 = -1;
     r.d1 = 0.f;
+    r.d2 = __int_as_float(0x7f800000);
     const u64 k1 = rk1[q], k2 = rk2[q];
     int i1 = -1, i2 = -1;
     float d1 = __int_as_float(0x7f800000), d2 = d1;
@@ -178,17 +180,21 @@ __device__ __forceinline__ RowResult eval_rows_win(const FinalizeParams& p, u64 
         pass = has1 && (no_ratio || (has2 && (double)d1 < p.ratio * (double)d2));
         scan_a = pass;
     } else if (has1) {
-        // the sweep ranked 1/2 d^2 in expansion form (error ~4e-7 absolute, or e): decide far-from-the-boundary rows on those values,
-        // evaluate the rest -- and every reported distance -- in direct form.  (A fast-mode row never lands in between: win_classify
-        // has sent those to the fallback sweep.)
+        // CHAIN keys: k1 = the best chain of 8 columns (its maximum is the row's best value s1), k2 = the second chain, whose value s2 is
+        // the best of every column outside the best chain.  The true second lies in one of the two chains, and s2 >= it: a certain fail
+        // on (s1, s2) is certain, a certain pass only says that the columns outside the best chain cannot fail the row -- the best
+        // chain's own second, evaluated below, must pass the exact test too.  No second chain (the train frame fits one chain, or every
+        // other chain is pad): s2 = +inf, and the best chain's own second decides.  The sweep's values are within ~4e-7 absolute of the
+        // expansion form (or within e): decide far-from-the-boundary rows on them, evaluate the rest -- and every reported distance --
+        // in direct form.  (A fast-mode row never lands in between: win_classify has sent those to the fallback sweep.)
         const float s1 = __uint_as_float((uint32_t)(k1 >> 32)), s2 = has2 ? __uint_as_float((uint32_t)(k2 >> 32)) : inf;
         if (no_ratio) { pass = true; scan_a = true; }
-        else if (has2 && p.ratio > 0.0) {
+        else if (p.ratio > 0.0) {
             const int cls = win_ratio_class(s1, s2, e, (float)(p.ratio * p.ratio));
             if (cls != 0) {
                 scan_a = true;
                 pass = cls == 1;
-                if (cls == 2) { scan_b = true; exact_ratio = true; }
+                if (cls == 2) { scan_b = true; exact_ratio = true; }     // (s2 = +inf is never class 2: has2 holds here)
             }
         }
         if (scan_b && a0 >= b0 && a1 <= b1) scan_a = false;       // slice a lies inside slice b: one evaluation
@@ -266,13 +272,16 @@ __device__ __forceinline__ RowResult eval_rows_win(const FinalizeParams& p, u64 
     if (KIND == ESFM_KIND_B256) {
         if (i1 < 0) pass = false;               // (cannot happen for a passing row: the sweep saw this distance in this slice)
     } else {
+        // class 2: the exact top 2 of both chains; class 1: the best chain's own second (none: the second chain, which cannot fail)
         if (exact_ratio) pass = i2 >= 0 && (double)d1 < p.ratio * (double)d2;
+        else if (pass && !no_ratio) pass = i2 >= 0 ? (double)d1 < p.ratio * (double)d2 : has2;
         if (i1 < 0) pass = false;
     }
     RowResult r;
     r.keep = pass;
     r.t1 = i1;
     r.d1 = d1;
+    r.d2 = i2 >= 0 ? d2 : inf;
     return r;
 }
 
@@ -386,10 +395,20 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
             if (p.phase == 1) {
                 // Who could beat a survivor (q, t) at its own train row t?  A row whose NEAREST train row is t (another survivor: settled by
                 // the claims below; a row that failed the ratio test: counted in histogram A by its best value), or a row for which t is at
-                // best second (then its second-best value is <= its distance to t: histogram B, every row).  A survivor whose distance
-                // lies below every such value needs no verification sweep.  Fast-mode values enter as lower bounds, value - e: the k-th
-                // smallest of a row's values moves by at most e, whichever column the sweep named.
-                if (k2 != kKeyInit) atomicAdd(&s_hist[1][fin_bucket<KIND>(__uint_as_float((uint32_t)(k2 >> 32)) - e)], 1u);
+                // best second (then its second-best value is <= its distance to t: histogram B takes a lower bound on every row's second
+                // value).  A survivor whose distance lies below every such value needs no verification sweep.  Fast-mode values enter as
+                // lower bounds, value - e: the k-th smallest of a row's values moves by at most e, whichever column the sweep named.
+                // SURF chain keys: k2 is the best value OUTSIDE the best chain, so k2 - e bounds the true second only from above when the
+                // second lies inside the best chain.  A survivor had its best chain evaluated exactly: its B entry is min(that chain's own
+                // second, k2 - e).  A row that did not survive enters histogram A at k1 - e, below its second value: the prefix test
+                // below only asks whether any entry lies at or below a value, so its B entry, never lower than its A entry, is dropped.
+                if (KIND == ESFM_KIND_B256) {
+                    if (k2 != kKeyInit) atomicAdd(&s_hist[1][fin_bucket<KIND>(__uint_as_float((uint32_t)(k2 >> 32)) - e)], 1u);
+                } else if (r.keep) {
+                    float lo2 = 0.5f * r.d2 * r.d2;     // (+inf: none)
+                    if (k2 != kKeyInit) lo2 = fminf(lo2, __uint_as_float((uint32_t)(k2 >> 32)) - e);
+                    if (lo2 != __int_as_float(0x7f800000)) atomicAdd(&s_hist[1][fin_bucket<KIND>(lo2)], 1u);
+                }
                 if (!r.keep && k1 != kKeyInit) atomicAdd(&s_hist[0][fin_bucket<KIND>(__uint_as_float((uint32_t)(k1 >> 32)) - e)], 1u);
                 // every train row some survivor points at is claimed by the nearest such query row (lowest index on ties)
                 if (r.keep) atomicMin(const_cast<u64*>(ck1) + r.t1, make_key(__float_as_uint(r.d1), (uint32_t)q));
@@ -517,8 +536,10 @@ __global__ void __launch_bounds__(kFinThreads) win_classify_kernel(const Finaliz
         int* gl = p.gather + (size_t)pair * p.stride;
         for (int q = threadIdx.x; q < fq; q += kFinThreads) {
             const u64 k1 = rk1[q], k2 = rk2[q];
-            if (k1 == kKeyInit || k2 == kKeyInit) continue;          // no second column: nothing to rank
-            const float s1 = __uint_as_float((uint32_t)(k1 >> 32)), s2 = __uint_as_float((uint32_t)(k2 >> 32));
+            if (k1 == kKeyInit) continue;                             // no column at all
+            // no second chain: s2 = +inf, settled -- the best chain holds every column, and finalize evaluates it exactly
+            const float s1 = __uint_as_float((uint32_t)(k1 >> 32));
+            const float s2 = k2 == kKeyInit ? __int_as_float(0x7f800000) : __uint_as_float((uint32_t)(k2 >> 32));
             const float e = win_fast_eps(row_eps[q], nq, nt);
             const bool unsettled = no_ratio ? !(s2 - s1 > 2.f * e) : win_ratio_class(s1, s2, e, r2) == 2;
             if (unsettled) gl[atomicAdd(&s_cnt, 1u)] = q;

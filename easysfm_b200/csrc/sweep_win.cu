@@ -4,18 +4,19 @@
 // Same contract towards the caller as the other sweeps (cpp_code/src/feature_matching.cpp:71-92 / :115-137 as exact brute force,
 // python_code/feature_match.py:26-27,33-39): per image pair the two nearest train rows of every query row and the nearest query
 // row of every train row, with OpenCV's lowest-index tie-break.  What differs is HOW a row's neighbours are reported:
-//     row key    = value bits << 32 | SLICE,    slice = (first column / 8) << 1 | wide: the 8 (SURF, best value) or 32 train columns
-//                                               the value was found in
+//     row key    = value bits << 32 | SLICE,    slice = (first column / 8) << 2 | width code: the 8, 32 or 64 train columns the value
+//                                               was found in (SURF: CHAIN keys, the best chain of 8 columns and the second chain of 8)
 //     column key = value bits << 32 | query row                                                    (unchanged)
-// finalize.cu finds the column inside the window by re-evaluating its 32 distances exactly (direct-form L2 / XOR + POPC), which it
+// finalize.cu finds the column inside the window by re-evaluating its distances exactly (direct-form L2 / XOR + POPC), which it
 // only does for the rows that can pass the ratio test.  The epilogue therefore needs VALUES only:
 //   * SURF (KIND = ESFM_KIND_F32X64, "H" split of tc_layout.cuh): 12 x tcgen05.mma.kind::f16 (a = fp16(x), b = fp16(x - a);
 //     b_q.a_t + a_q.b_t + a_q.a_t, fp32 accumulation; fp16 subnormals are honoured by the tensor core: h16_probe.cu) + the exact
 //     kind::tf32 half-norm step = 13 MMA slots per 128 x 128 tile instead of 25, tile image 36 KB instead of 68 KB.  FAST mode
 //     (SweepParams::win_fast, the rows-only sweep's default) drops b_q: 8 + 1 = 9 slots, values within win_fast_eps (esfm_internal.cuh);
 //     the rows that bound cannot settle are swept again in exact mode (SweepParams::fallback, finalize.cu win_classify_kernel).  Epilogue:
-//     a branch-free tournament over the 32 accumulators of a pass gives the pass's two largest -1/2 d^2, eleven selects merge them
-//     into the running (k1, w1, k2, w2).
+//     chain keys -- the maximum of every chain of 8 columns (FMNMX3), the two largest of a unit's 8 chain maxima with their chains, merged
+//     into the running (k1, w1, k2, w2): ~1.2 ALU instructions per comparison instead of ~3 for an exact per-row top 2.  The row's true
+//     second lies in its best chain or is its second chain's maximum; finalize evaluates the best chain exactly and learns the rest.
 //   * ORB (KIND = ESFM_KIND_B256): the +-1 FP8 operands of sweep_l2_tc.cu with FP16 ACCUMULATORS (-2 hamming, exact; pad rows
 //     overflow to -inf): tcgen05.ld.pack::16b delivers two columns per register and the whole epilogue runs on packed halves
 //     (HMNMX2 / VHMNMX tournament, HFMA2.RELU threshold tests): ~1/2 the instructions per element of the fp32 epilogue.
@@ -32,7 +33,7 @@
 //   warps 0-15   epilogue in four GROUPS of four warps (one per TMEM lane quarter = 32 query rows).  The unit of work is half a tile
 //                (64 train columns): unit 2 g + h belongs to group (2 g + h) % 4, so a group reads one half of every other tile -- ORB: 32
 //                packed registers in one tcgen05.ld; SURF: two loads of 32 -- releases its share of the accumulator stage BEFORE it
-//                computes, and runs one tournament over its columns: twice the columns per barrier hand-shake and per running-state
+//                computes, and runs one selection over its columns: twice the columns per barrier hand-shake and per running-state
 //                merge of a 32-column pass, and a slow warp delays nobody else's stage.
 // Every mbarrier keeps ONE producer and ONE consumer role (a parity wait may not skip a phase): the barriers of the load ring are indexed
 // by tile % lcm(5 stages, 3 issuers) = 15, those of the accumulator ring by tile % lcm(3 stages, 3 issuers, 4 groups) = 12.
@@ -82,7 +83,7 @@ __device__ __forceinline__ void tmem_ld32_pack(uint32_t taddr, uint32_t (&v)[32]
         : "memory");
 }
 
-// merge the pass's two largest values (p1 >= p2, found in the column slices id1 / id2) into the running (k1, w1, k2, w2): strict
+// merge a unit's two largest values (p1 >= p2, found in the column slices id1 / id2) into the running (k1, w1, k2, w2): strict
 // comparisons, so of equal values the one found first (the lower slice = the lower column) stays in front
 __device__ __forceinline__ void win_merge(float p1, int id1, float p2, int id2, float& k1, int& w1, float& k2, int& w2) {
     const bool c1 = p1 > k1;
@@ -411,8 +412,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_win_kernel(const SweepPar
                         const int sub = pm0 == p1 ? 0 : 1;                  // the lower part on ties
                         if (!(p.debug_flags & 16)) win_merge(p1, win_slice(c0 + 32 * sub, 1), p2, win_slice(c0, 2), k1, w1, k2, w2);
                     } else {
-                        // ---------------- SURF: two quarters of 32 fp32 accumulators v = -1/2 d^2 (pads: <= -1e30) ----------------
-#pragma unroll 1
+                        // ---------------- SURF: 64 fp32 accumulators v = -1/2 d^2 (pads: <= -1e30), loaded 32 at a time ----------------
+                        // Chain keys: of every chain of 8 columns only its maximum is kept, and the row keeps the two largest chain maxima
+                        // with their chains.  The best column lies in the best chain; the true second lies in the best chain or is the
+                        // maximum of the second chain; finalize.cu evaluates the best chain exactly and so learns its own second.
+                        float m[8];
+#pragma unroll
                         for (int qc = 0; qc < 2; ++qc) {
                             uint32_t vb[32];
                             tmem_ld32(tmem + lane_addr + as * 128 + half * 64 + qc * 32, vb);
@@ -422,33 +427,30 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_win_kernel(const SweepPar
                                 __syncwarp();
                                 if (lane == 0) mbar_arrive_relaxed(&accEmpty[ab]);
                             }
-                            if (p.debug_flags & 1) continue;
-                            float v[32];
 #pragma unroll
-                            for (int c = 0; c < 32; ++c) v[c] = __uint_as_float(vb[c]);
-                            // in-place tournament: sorted pairs, merged down to one (largest, second) per chain of 8 columns: v[8 j], v[8 j + 1]
-#pragma unroll
-                            for (int j = 0; j < 16; ++j) {
-                                const float hi = fmaxf(v[2 * j], v[2 * j + 1]), lo = fminf(v[2 * j], v[2 * j + 1]);
-                                v[2 * j] = hi; v[2 * j + 1] = lo;
+                            for (int j = 0; j < 4; ++j) {
+                                const float* v = reinterpret_cast<const float*>(vb) + 8 * j;
+                                m[4 * qc + j] = fmaxf(fmaxf(fmaxf(v[0], v[1]), v[2]), fmaxf(fmaxf(fmaxf(v[3], v[4]), v[5]), fmaxf(v[6], v[7])));
                             }
-#pragma unroll
-                            for (int step = 1; step < 4; step <<= 1) {
-#pragma unroll
-                                for (int j = 0; j < 16; j += 2 * step) {
-                                    const float ha = v[2 * j], la = v[2 * j + 1], hc = v[2 * (j + step)], lc = v[2 * (j + step) + 1];
-                                    v[2 * j] = fmaxf(ha, hc);
-                                    v[2 * j + 1] = fmaxf(fmaxf(fminf(ha, hc), la), lc);
-                                }
-                            }
-                            const float h01 = fmaxf(v[0], v[8]), l01 = fmaxf(fmaxf(fminf(v[0], v[8]), v[1]), v[9]);
-                            const float h23 = fmaxf(v[16], v[24]), l23 = fmaxf(fmaxf(fminf(v[16], v[24]), v[17]), v[25]);
-                            const float p1 = fmaxf(h01, h23), p2 = fmaxf(fmaxf(fminf(h01, h23), l01), l23);
-                            // the best value's chain of 8 columns (the lowest on ties): finalize evaluates 8 candidates instead of 32
-                            const int sub = v[0] == p1 ? 0 : (v[8] == p1 ? 1 : (v[16] == p1 ? 2 : 3));
-                            const int cq = c0 + qc * 32;
-                            if (!(p.debug_flags & 16)) win_merge(p1, win_slice(cq + 8 * sub, 0), p2, win_slice(cq, 1), k1, w1, k2, w2);
                         }
+                        if (p.debug_flags & (1 | 16)) continue;
+                        // the two largest chain maxima (values: sorted pairs, merged), then the best chain, the lowest one on ties
+                        const float h01 = fmaxf(m[0], m[1]), l01 = fminf(m[0], m[1]), h23 = fmaxf(m[2], m[3]), l23 = fminf(m[2], m[3]);
+                        const float h45 = fmaxf(m[4], m[5]), l45 = fminf(m[4], m[5]), h67 = fmaxf(m[6], m[7]), l67 = fminf(m[6], m[7]);
+                        const float ha = fmaxf(h01, h23), la = fmaxf(fmaxf(fminf(h01, h23), l01), l23);
+                        const float hb = fmaxf(h45, h67), lb = fmaxf(fmaxf(fminf(h45, h67), l45), l67);
+                        const float p1 = fmaxf(ha, hb), p2 = fmaxf(fmaxf(fminf(ha, hb), la), lb);
+                        int j1 = 7;
+#pragma unroll
+                        for (int j = 6; j >= 0; --j) j1 = m[j] == p1 ? j : j1;
+                        // The second chain's index is read only where both chains beat the running best (p2 > k1, win_merge): the first
+                        // units of a row, rarely any later one, so it is found on a warp-uniform branch.  Lowest chain other than j1 on ties.
+                        int j2 = 0;
+                        if (__any_sync(0xffffffffu, p2 > k1)) {
+#pragma unroll
+                            for (int j = 7; j >= 0; --j) j2 = (m[j] == p2 && j != j1) ? j : j2;
+                        }
+                        win_merge(p1, win_slice(c0 + 8 * j1, 0), p2, win_slice(c0 + 8 * j2, 0), k1, w1, k2, w2);
                     }
                 }
                 // ---- end of the sweep for this query block: merge the four groups' results of every row (64-bit shared-memory atomics on
