@@ -258,7 +258,6 @@ extern "C" int esfm_init(int device, void* cuda_stream, esfm_ctx_t** out) {
     ctx->device = device;
     ctx->sm_count = prop.multiProcessorCount;
     if (const char* z = getenv("ESFM_ORB_Z")) ctx->orb_z = atoi(z) != 0;
-    if (const char* z = getenv("ESFM_TWO_PHASE")) ctx->two_phase = atoi(z) != 0;
     if (const char* z = getenv("ESFM_TC16_EXACT")) ctx->tc16_exact = atoi(z) != 0;
     if (const char* eng = getenv("ESFM_HAMMING_ENGINE")) {
         if (!strcmp(eng, "tc") || !strcmp(eng, "tensor")) ctx->hamming_engine = ESFM_HAMMING_ENGINE_TC;
@@ -765,16 +764,56 @@ struct ChunkPlan {
     size_t chunk_pairs;
 };
 
-// any tensor-core sweep (they share the scratch layout: column thresholds, one query tile per block)
-bool use_tc(const esfm_ctx* ctx, const esfm_bank* b) {
-    return b->kind == ESFM_KIND_F32X64 ? ctx->l2_engine != ESFM_L2_ENGINE_FFMA : ctx->hamming_engine != ESFM_HAMMING_ENGINE_POPC;
-}
-// the 16-bit sweeps of sweep_win.cu (row keys carry a slice of columns)
-bool use_win(const esfm_ctx* ctx, const esfm_bank* b) {
-    return b->kind == ESFM_KIND_F32X64 ? ctx->l2_engine == ESFM_L2_ENGINE_TC16 : ctx->hamming_engine == ESFM_HAMMING_ENGINE_TC16;
+// The sweep kernels: sweep_l2.cu, sweep_hamming.cu, sweep_l2_tc.cu (rows and column minima in one sweep), sweep_win.cu (rows only, slice keys)
+enum class SweepKind { Ffma, Popc, Tc, Win };
+
+// How one chunk is swept: the kernel, what it needs from the bank and the scratch, and how finalize reads its keys
+struct SweepPlan {
+    SweepKind sweep;
+    TcImage image;                              // operand image of the bank (Tc, Win)
+    int thr_fill = -1;                          // byte the column thresholds start at; -1: the sweep reads none
+    KeyFormat key_format = KeyFormat::Direct;
+    bool fast;           // SURF Win: fast mode, then an exact fallback sweep of the rows its error bound cannot settle
+    bool two_phase;      // Win cross-check: ratio test, then a verification sweep of the undecided train rows (finalize.cu)
+};
+
+// The tc16 sweeps (sweep_win.cu) are ROWS-ONLY.  Their cross-check runs in TWO PHASES: (1) the rows-only sweep + ratio test, survivors
+// claim their train rows and histograms of every row's best / second-best value decide which survivors could still be beaten; (2) a
+// second rows-only sweep with the roles swapped over just the undecided train rows (gathered into the query operand), whose answer --
+// the nearest query row of each -- settles them.  Raw knn output (esfm_knn2_pair) needs column minima inside ONE sweep: a tc16 context
+// runs it on the fp32-accumulator sweep of sweep_l2_tc.cu (the bank's operand image is rebuilt on the switch).
+SweepPlan plan_sweep(const esfm_ctx* ctx, const esfm_bank* b, bool cross_check, bool knn) {
+    const bool surf = b->kind == ESFM_KIND_F32X64;
+    const int engine = surf ? ctx->l2_engine : ctx->hamming_engine;
+    SweepPlan s{};
+    if (engine == (surf ? ESFM_L2_ENGINE_FFMA : ESFM_HAMMING_ENGINE_POPC)) {
+        s.sweep = surf ? SweepKind::Ffma : SweepKind::Popc;
+        if (surf) s.thr_fill = kThrInit & 0xff;      // (the POPC sweep keeps its column minima in shared memory)
+    } else if (engine == (surf ? ESFM_L2_ENGINE_TC16 : ESFM_HAMMING_ENGINE_TC16) && !knn) {
+        s.sweep = SweepKind::Win;                     // (col_thr only holds its gather lists)
+        s.image = surf ? TcImage::H : TcImage::Fp8Pm1;
+        s.key_format = KeyFormat::Slice;
+        s.fast = surf && !ctx->tc16_exact;
+        s.two_phase = cross_check;
+    } else {
+        s.sweep = SweepKind::Tc;
+        if (surf) {
+            s.image = TcImage::Tf32x3;
+            s.thr_fill = kTcBoundBitsF32 & 0xff;
+        } else if (ctx->orb_z && b->max_rows <= kTcZMaxRows) {     // the column index rides in the Z key: at most 2^15 rows per frame
+            s.image = TcImage::Fp8Z;
+            s.thr_fill = kTcBoundBitsZ & 0xff;
+            s.key_format = KeyFormat::TcZ;
+        } else {
+            s.image = TcImage::Fp8Pm1;
+            s.thr_fill = kTcBoundBitsB256 & 0xff;
+            s.key_format = KeyFormat::TcPm1;
+        }
+    }
+    return s;
 }
 
-ChunkPlan plan_chunks(const esfm_bank* b, int64_t n_pairs, bool split_for_overlap = false) {
+ChunkPlan plan_chunks(const esfm_bank* b, int64_t n_pairs) {
     ChunkPlan pl;
     const int padded = ((b->max_rows + kTile - 1) / kTile) * kTile;
     pl.stride = std::max(padded, kTile);
@@ -783,23 +822,22 @@ ChunkPlan plan_chunks(const esfm_bank* b, int64_t n_pairs, bool split_for_overla
     const size_t arena_bytes_per_pair = (size_t)std::max(b->max_rows, 1) * sizeof(esfm_dmatch_t);
     const size_t budget_keys = (size_t)4 << 30, budget_arena = (size_t)2 << 30;
     size_t c = std::min(budget_keys / key_bytes_per_pair, budget_arena / arena_bytes_per_pair);
-    c = std::max<size_t>(1, std::min<size_t>(c, 65536));
-    if (const char* e = getenv("ESFM_CHUNK_PAIRS")) c = std::max<size_t>(1, std::min<size_t>(c, (size_t)atoll(e)));   // tests: force several chunks
     // (Measured: splitting a batch that fits in one or two chunks into four equal ones to overlap more of the match download LOSES -- ORB e2e
     // 3.99e12 -> 3.38e12 comparisons/s: per-chunk launches, synchronisations and the pinned-slot streaming cost more than the exposed copy.)
-    (void)split_for_overlap;
+    c = std::max<size_t>(1, std::min<size_t>(c, 65536));
+    if (const char* e = getenv("ESFM_CHUNK_PAIRS")) c = std::max<size_t>(1, std::min<size_t>(c, (size_t)atoll(e)));   // tests: force several chunks
     pl.chunk_pairs = (size_t)std::min<int64_t>((int64_t)c, std::max<int64_t>(n_pairs, 1));
     return pl;
 }
 
-int ensure_scratch(esfm_ctx* ctx, const esfm_bank* b, const ChunkPlan& pl, int n_bufs) {
+int ensure_scratch(esfm_ctx* ctx, const esfm_bank* b, const SweepPlan& sw, const ChunkPlan& pl, int n_bufs) {
     size_t key_elems = pl.chunk_pairs * 4 * (size_t)pl.stride;
     size_t cap = ctx->keys_bytes / sizeof(u64);
     if (int rc = grow(&ctx->keys, &cap, key_elems)) return rc;
     ctx->keys_bytes = cap * sizeof(u64);
-    if (b->kind == ESFM_KIND_F32X64 || use_tc(ctx, b))
+    if (sw.sweep != SweepKind::Popc)
         if (int rc = grow(&ctx->col_thr, &ctx->col_thr_elems, pl.chunk_pairs * (size_t)pl.stride)) return rc;
-    if (use_win(ctx, b))
+    if (sw.sweep == SweepKind::Win)
         if (int rc = grow(&ctx->gather_cnt, &ctx->gather_cnt_elems, pl.chunk_pairs)) return rc;
     const size_t arena_need = pl.chunk_pairs * (size_t)std::max(b->max_rows, 1);
     for (int k = 0; k < n_bufs; ++k) {
@@ -843,18 +881,17 @@ int ensure_kmajor_layout(esfm_ctx* ctx, esfm_bank* b) {
     return ESFM_OK;
 }
 
-// Tensor-core engines: the operand images of tc_layout.cuh.  z_mode: F32X64: 0 = 3xTF32 hi/lo images, 2 = the 16-bit split ("H")
-// images of sweep_win.cu; B256: 0 = +-1 FP8 images (also what sweep_win.cu reads), 1 = "Z" encoding.
+// Tensor-core engines: the operand images of tc_layout.cuh (TcImage).
 // The H images are followed by what win_fast_eps needs: float row_eps[total rows], frame_norm[n_frames].
 float* tch_row_eps(const esfm_bank* b) { return reinterpret_cast<float*>(b->d_tc + ((size_t)b->tile_off[b->n_frames] + 1) * kTchTileBytes); }
 float* tch_frame_norm(const esfm_bank* b) { return tch_row_eps(b) + b->row_off[b->n_frames]; }
 
-int ensure_tc_layout(esfm_ctx* ctx, esfm_bank* b, int z_mode) {
-    if (b->tc_built && b->tc_z == z_mode) return ESFM_OK;
-    b->tc_z = z_mode;
+int ensure_tc_layout(esfm_ctx* ctx, esfm_bank* b, TcImage img) {
+    if (b->tc_built && b->tc_image == img) return ESFM_OK;
+    b->tc_image = img;
     const int n_tiles = b->tile_off[b->n_frames];
-    b->tc_bytes = ((size_t)n_tiles + 1) * (b->kind == ESFM_KIND_F32X64 && z_mode != 2 ? (size_t)kTcTileBytes : (size_t)kTc8TileBytes);
-    if (b->kind == ESFM_KIND_F32X64 && z_mode == 2) b->tc_bytes += ((size_t)b->row_off[b->n_frames] + b->n_frames) * sizeof(float);
+    b->tc_bytes = ((size_t)n_tiles + 1) * (img == TcImage::Tf32x3 ? (size_t)kTcTileBytes : (size_t)kTc8TileBytes);
+    if (img == TcImage::H) b->tc_bytes += ((size_t)b->row_off[b->n_frames] + b->n_frames) * sizeof(float);
     if (!b->d_tc || b->tc_cap < b->tc_bytes) {
         if (b->d_tc) cudaFreeAsync(b->d_tc, ctx->stream);   // (stream-ordered: earlier sweeps have been enqueued before)
         b->d_tc = nullptr;
@@ -862,52 +899,35 @@ int ensure_tc_layout(esfm_ctx* ctx, esfm_bank* b, int z_mode) {
         if (e != cudaSuccess) { cudaGetLastError(); return fail(ESFM_ERR_NOMEM, "cudaMallocAsync(%zu) for the tensor-core bank failed: %s", b->tc_bytes, cudaGetErrorString(e)); }
         b->tc_cap = b->tc_bytes;
     }
-    cudaError_t e = b->kind == ESFM_KIND_F32X64
-            ? (z_mode == 2 ? launch_pack_tch((const float*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc,
-                                             tch_row_eps(b), tch_frame_norm(b), ctx->stream)
-                           : launch_pack_tc((const float*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc, ctx->stream))
-            : launch_pack_tc8((const uint32_t*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc, z_mode, ctx->stream);
+    cudaError_t e =
+        img == TcImage::H ? launch_pack_tch((const float*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc,
+                                            tch_row_eps(b), tch_frame_norm(b), ctx->stream)
+        : img == TcImage::Tf32x3 ? launch_pack_tc((const float*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc, ctx->stream)
+        : launch_pack_tc8((const uint32_t*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, n_tiles, b->d_tc,
+                          img == TcImage::Fp8Z ? 1 : 0, ctx->stream);
     if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "tensor-core pack kernel launch failed: %s", cudaGetErrorString(e));
     if (n_tiles > 0) ctx->stats.kernel_launches += 1;
     b->tc_built = true;
     return ESFM_OK;
 }
 
-int units_per_pair(const esfm_ctx* ctx, const esfm_bank* b, size_t n_chunk_pairs) {
+int units_per_pair(const esfm_ctx* ctx, const esfm_bank* b, const SweepPlan& sw, size_t n_chunk_pairs) {
     if (n_chunk_pairs >= (size_t)4 * ctx->sm_count) return 1;
-    const int qblock_rows = use_tc(ctx, b) ? kTile : (b->kind == ESFM_KIND_F32X64 ? kQTiles * kTile : kConsumerThreads * kHamRQ);
+    const int qblock_rows = sw.sweep == SweepKind::Ffma ? kQTiles * kTile : (sw.sweep == SweepKind::Popc ? kConsumerThreads * kHamRQ : kTile);
     const int max_blocks = std::max(1, (b->max_rows + qblock_rows - 1) / qblock_rows);
     const int want = (int)((4 * (size_t)ctx->sm_count + n_chunk_pairs - 1) / std::max<size_t>(n_chunk_pairs, 1));
     return std::max(1, std::min(want, max_blocks));
 }
 
 // Enqueues sweep + finalize for one chunk that is already described in cb.d_pairs (compute stream only).
-int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, size_t n, double ratio, int cross_check, int32_t* knn_idx,
-              float* knn_dist) {
-    CUDA_TRY(cudaMemsetAsync(ctx->keys, 0xFF, n * 4 * (size_t)pl.stride * sizeof(u64), ctx->stream));
+int run_chunk(esfm_ctx* ctx, esfm_bank* b, const SweepPlan& sw, const ChunkPlan& pl, ChunkBuf& cb, size_t n, double ratio, int cross_check,
+              int32_t* knn_idx, float* knn_dist) {
+    CUDA_TRY(cudaMemsetAsync(ctx->keys, (int)(kKeyInit & 0xff), n * 4 * (size_t)pl.stride * sizeof(u64), ctx->stream));
     CUDA_TRY(cudaMemsetAsync(cb.d_cursor, 0, 3 * sizeof(unsigned long long), ctx->stream));
-    const bool tc = use_tc(ctx, b);
-    // ORB "Z" encoding: the column index rides in the key, so every frame must have at most 2^15 rows; else the +-1 encoding
-    // tc16 sweeps (sweep_win.cu) are ROWS-ONLY.  Their cross-check runs in TWO PHASES: (1) the rows-only sweep + ratio test, survivors claim
-    // their train rows and histograms of every row's best / second-best value decide which survivors could still be beaten; (2) a second
-    // rows-only sweep with the roles swapped over just the undecided train rows (gathered into the query operand), whose answer -- the
-    // nearest query row of each -- settles them.  What needs column minima inside ONE sweep (esfm_knn2_pair; $ESFM_TWO_PHASE=0) runs on the
-    // fp32-accumulator tensor-core sweep of sweep_l2_tc.cu instead (the bank's operand images are rebuilt on the switch).
-    const bool win_engine = tc && use_win(ctx, b);
-    const bool two_phase = win_engine && cross_check && !knn_idx && ctx->two_phase;
-    const bool win = win_engine && !knn_idx && (two_phase || !cross_check);
-    const int zmode = (tc && !win && b->kind == ESFM_KIND_B256 && ctx->orb_z && b->max_rows <= kTcZMaxRows) ? 1 : 0;
-    // SURF: the rows-only sweep runs in fast mode (9 MMA slots per tile); the rows its error bound leaves unsettled are re-swept exactly
-    const bool win_fast = win && b->kind == ESFM_KIND_F32X64 && !ctx->tc16_exact;
-    if (tc) { if (int rc = ensure_tc_layout(ctx, b, win && b->kind == ESFM_KIND_F32X64 ? 2 : zmode)) return rc; }
-    else if (b->kind == ESFM_KIND_F32X64) { if (int rc = ensure_kmajor_layout(ctx, b)) return rc; }
-    if ((b->kind == ESFM_KIND_F32X64 || tc) && !two_phase)
-        // column thresholds start at "no bound yet" (a repeated byte): FFMA engine 0x7f7f7f7f = 3.39e38f; tensor-core engines
-        // 0x6f6f6f6f = 7.4e28f for SURF (below its 1e30 pad-row norm), 0x47474747 = 51015f for ORB +-1 (above every real
-        // value, below the pad rows), 0x4b4b4b4b = 1.33e7f for ORB "Z" (above every key); the FP16-accumulator ORB sweep keeps
-        // fp16 thresholds: 0x6060 = 560 (above every 2 * hamming)
-        CUDA_TRY(cudaMemsetAsync(ctx->col_thr, tc ? (b->kind == ESFM_KIND_F32X64 ? 0x6F : (win ? 0x60 : (zmode ? 0x4B : 0x47))) : 0x7F,
-                                 n * (size_t)pl.stride * sizeof(uint32_t), ctx->stream));
+    if (sw.sweep == SweepKind::Tc || sw.sweep == SweepKind::Win) { if (int rc = ensure_tc_layout(ctx, b, sw.image)) return rc; }
+    else if (sw.sweep == SweepKind::Ffma) { if (int rc = ensure_kmajor_layout(ctx, b)) return rc; }
+    if (sw.thr_fill >= 0)
+        CUDA_TRY(cudaMemsetAsync(ctx->col_thr, sw.thr_fill, n * (size_t)pl.stride * sizeof(uint32_t), ctx->stream));
     SweepParams sp{};
     sp.kmajor = b->d_kmajor;
     sp.rows_f32 = (const float*)b->d_rows;
@@ -918,21 +938,20 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, si
     sp.frame_tile_off = b->d_tile_off;
     sp.pairs = cb.d_pairs;
     sp.n_pairs = (int)n;
-    sp.units_per_pair = units_per_pair(ctx, b, n);
+    sp.units_per_pair = units_per_pair(ctx, b, sw, n);
     sp.keys = ctx->keys;
     sp.col_thr = ctx->col_thr;
     sp.stride = pl.stride;
     sp.col_cap = pl.col_cap;
-    sp.need_cols = ((cross_check && !two_phase) || knn_idx) ? 1 : 0;
+    sp.need_cols = ((cross_check && !sw.two_phase) || knn_idx) ? 1 : 0;
     if (const char* dbg = getenv("ESFM_TC_DEBUG")) sp.debug_flags = atoi(dbg);
-    sp.tc_qtiles = 1;
-    sp.tc_kind = zmode ? kTcKindB256Z : b->kind;
-    sp.win_fast = win_fast ? 1 : 0;
+    sp.tc_kind = sw.image == TcImage::Fp8Z ? kTcKindB256Z : b->kind;
+    sp.win_fast = sw.fast ? 1 : 0;
     if (ctx->profiling) CUDA_TRY(cudaEventRecord(cb.ev_t0, ctx->stream));
-    cudaError_t e = win ? launch_sweep_win(sp, ctx->sm_count, ctx->stream)
-                  : tc ? launch_sweep_l2_tc(sp, ctx->sm_count, ctx->stream)
-                       : (b->kind == ESFM_KIND_F32X64 ? launch_sweep_l2(sp, ctx->sm_count, ctx->stream)
-                                                      : launch_sweep_hamming(sp, ctx->sm_count, ctx->stream));
+    cudaError_t e = sw.sweep == SweepKind::Win ? launch_sweep_win(sp, ctx->sm_count, ctx->stream)
+                  : sw.sweep == SweepKind::Tc ? launch_sweep_l2_tc(sp, ctx->sm_count, ctx->stream)
+                  : sw.sweep == SweepKind::Ffma ? launch_sweep_l2(sp, ctx->sm_count, ctx->stream)
+                                                : launch_sweep_hamming(sp, ctx->sm_count, ctx->stream);
     if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "sweep kernel launch failed: %s", cudaGetErrorString(e));
     FinalizeParams fp{};
     fp.kind = b->kind;
@@ -946,9 +965,8 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, si
     fp.stride = pl.stride;
     fp.ratio = ratio;
     fp.cross_check = cross_check ? 1 : 0;
-    fp.b256_float_keys = (tc && b->kind == ESFM_KIND_B256) ? (zmode ? 2 : 1) : 0;
-    fp.win_keys = win ? 1 : 0;
-    fp.phase = two_phase ? 1 : 0;
+    fp.key_format = sw.key_format;
+    fp.phase = sw.two_phase ? 1 : 0;
     fp.gather = reinterpret_cast<int*>(ctx->col_thr);
     fp.gather_cnt = ctx->gather_cnt;
     fp.arena = cb.arena;
@@ -959,7 +977,7 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, si
     fp.pair_cnt = cb.d_pair_cnt;
     fp.knn_idx = knn_idx;
     fp.knn_dist = knn_dist;
-    if (win_fast) {
+    if (sw.fast) {
         // rows the fast sweep cannot settle -> the pair's gather list -> one exact sweep of just those rows (sweep time)
         fp.row_eps = tch_row_eps(b);
         fp.frame_norm = tch_frame_norm(b);
@@ -978,8 +996,8 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const ChunkPlan& pl, ChunkBuf& cb, si
     if (ctx->profiling) CUDA_TRY(cudaEventRecord(cb.ev_t1, ctx->stream));
     e = launch_finalize(fp, ctx->stream);
     if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "finalize kernel launch failed: %s", cudaGetErrorString(e));
-    cb.two_phase = two_phase;
-    if (two_phase) {
+    cb.two_phase = sw.two_phase;
+    if (sw.two_phase) {
         SweepParams vp = sp;
         vp.gather = fp.gather;
         vp.gather_cnt = fp.gather_cnt;
@@ -1076,10 +1094,11 @@ int esfm::match_pairs_impl(esfm_bank* b, const esfm_pair_t* pairs, int64_t n_pai
     }
     if (n_pairs == 0) { guard.r = nullptr; *out = res; return ESFM_OK; }
 
-    const ChunkPlan pl = plan_chunks(b, n_pairs, opts.fetch);       // (a device-resident batch must stay one chunk if it can)
+    const SweepPlan sw = plan_sweep(ctx, b, cross_check != 0, false);
+    const ChunkPlan pl = plan_chunks(b, n_pairs);
     const size_t n_chunks = ((size_t)n_pairs + pl.chunk_pairs - 1) / pl.chunk_pairs;
     const bool streamed = opts.fetch && (n_chunks > 1 || digests_only);   // matches go to pageable memory through the pinned slots
-    if (int rc = ensure_scratch(ctx, b, pl, n_chunks > 1 ? 2 : 1)) return rc;
+    if (int rc = ensure_scratch(ctx, b, sw, pl, n_chunks > 1 ? 2 : 1)) return rc;
 
     struct Chunk { size_t c0 = 0, n = 0; std::vector<uint32_t> order; };
     Chunk chunks[2];
@@ -1106,7 +1125,7 @@ int esfm::match_pairs_impl(esfm_bank* b, const esfm_pair_t* pairs, int64_t n_pai
         }
         CUDA_TRY(cudaMemcpyAsync(cb.d_pairs, cb.h_pairs, ch.n * sizeof(PairDesc), cudaMemcpyHostToDevice, ctx->stream));
         ctx->stats.h2d_bytes += ch.n * sizeof(PairDesc);
-        return run_chunk(ctx, b, pl, cb, ch.n, ratio, cross_check, nullptr, nullptr);
+        return run_chunk(ctx, b, sw, pl, cb, ch.n, ratio, cross_check, nullptr, nullptr);
     };
     auto enqueue_meta = [&](size_t k) -> int {      // counts + offsets + cursor of chunk k -> pinned host memory (copy stream)
         Chunk& ch = chunks[k & 1];
@@ -1367,8 +1386,9 @@ extern "C" int esfm_knn2_pair(esfm_bank_t* b, int query_frame, int train_frame, 
     if (int rc = set_device(ctx)) return rc;
     const int fq = b->rows[query_frame];
     if (fq == 0) return ESFM_OK;
+    const SweepPlan sw = plan_sweep(ctx, b, false, true);
     const ChunkPlan pl = plan_chunks(b, 1);
-    if (int rc = ensure_scratch(ctx, b, pl, 1)) return rc;
+    if (int rc = ensure_scratch(ctx, b, sw, pl, 1)) return rc;
     ChunkBuf& cb = ctx->buf[0];
     int32_t* d_idx = nullptr;
     float* d_dist = nullptr;
@@ -1380,7 +1400,7 @@ extern "C" int esfm_knn2_pair(esfm_bank_t* b, int query_frame, int train_frame, 
     int rc = ESFM_OK;
     e = cudaMemcpyAsync(cb.d_pairs, cb.h_pairs, sizeof(PairDesc), cudaMemcpyHostToDevice, ctx->stream);
     if (e != cudaSuccess) rc = fail(ESFM_ERR_CUDA, "cudaMemcpyAsync failed: %s", cudaGetErrorString(e));
-    if (!rc) rc = run_chunk(ctx, b, pl, cb, 1, 0.0, 0, d_idx, d_dist);
+    if (!rc) rc = run_chunk(ctx, b, sw, pl, cb, 1, 0.0, 0, d_idx, d_dist);
     if (!rc) {
         e = cudaMemcpyAsync(idx, d_idx, (size_t)fq * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);
         if (e == cudaSuccess) e = cudaMemcpyAsync(dist, d_dist, (size_t)fq * 2 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);

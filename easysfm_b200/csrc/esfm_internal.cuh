@@ -39,6 +39,23 @@ constexpr int kTcZMaxRows = 1 << kTcZShift;          // frames with more rows us
 constexpr int kTcZ0i = 21 * 448 * 448 - (1 << 22);   // 20480: what the 21 offset slots leave after cancelling -2^22
 constexpr int kHamIdxBits = 20;                      // packed 32-bit key = dist << 20 | index  (rows per frame < 2^20)
 
+// "No bound yet" of the running column thresholds: above every real value, below the pad rows.  FFMA sweep: 3.39e38f.  Tensor-core
+// sweeps: SURF 7.4e28 (pads: 1e30), ORB 51015 (real 2 * hamming <= 512, pads >= 200704), ORB "Z" 1.33e7 (keys < 2^24).
+constexpr uint32_t kThrInit = 0x7f7f7f7fu;
+constexpr uint32_t kTcBoundBitsF32 = 0x6f6f6f6fu, kTcBoundBitsB256 = 0x47474747u, kTcBoundBitsZ = 0x4b4b4b4bu;
+// cudaMemsetAsync writes the thresholds' start value, so each sentinel must be one byte repeated
+__host__ __device__ constexpr bool is_byte_fill(uint32_t v) { return v == (v & 0xffu) * 0x01010101u; }
+static_assert(is_byte_fill(kThrInit) && is_byte_fill(kTcBoundBitsF32) && is_byte_fill(kTcBoundBitsB256) && is_byte_fill(kTcBoundBitsZ),
+              "column-threshold sentinels must be a repeated byte");
+
+// How finalize reads the row and column keys a sweep leaves (FinalizeParams::key_format):
+//   Direct  key = (distance bits << 32) | column, high word read as it is: the POPC sweep's integer Hamming distance, 1/2 d^2 of the SURF
+//           ffma and tc sweeps (re-evaluated in direct form anyway);
+//   TcPm1   ORB tc sweep, +-1 encoding: high word = the float 2 * hamming;
+//   TcZ     ORB tc sweep, "Z" encoding: high word = the float z = kTcZ0i + 2^15 * hamming + column (tc_layout.cuh);
+//   Slice   sweep_win.cu (both kinds): row keys name a slice of train columns instead of a column (see finalize.cu).
+enum class KeyFormat : int { Direct, TcPm1, TcZ, Slice };
+
 struct PairDesc {
     int32_t q_frame, t_frame;
 };
@@ -63,7 +80,6 @@ struct SweepParams {
     int col_cap;                // Hamming sweep: smem column-minimum capacity in entries
     int tc_kind;                // TC sweeps: ESFM_KIND_F32X64 (3xTF32 L2; sweep_win: 16-bit split), ESFM_KIND_B256 (FP8 Hamming) or kTcKindB256Z (FP8 Hamming, packed
                                 // (distance, column) keys from the MMA); tc_main holds that kind's images
-    int tc_qtiles;              // TC sweep geometry: query tiles per block (always 1: the two-tile variant of round 1 is no longer built)
     int need_cols;              // 0: cross_check is off, nobody reads the column minima -- the tensor-core sweeps skip the column side
     // sweep_win.cu, verification pass of the two-phase cross-check: the query operand is a GATHERED subset of the pair's TRAIN frame
     // (gather[pair * stride + slot] = row of the train frame, gather_cnt[pair] rows), swept against the pair's QUERY frame; the best
@@ -99,9 +115,7 @@ struct FinalizeParams {
     unsigned long long* pair_off;  // [n_pairs] offset of each pair's matches in the arena
     int32_t* pair_cnt;          // [n_pairs]
     int* overflow;              // set to 1 if the arena was too small
-    int b256_float_keys;        // B256 keys from the tensor-core sweeps: 1 = high word is the float bits of 2 * hamming, 2 = of the packed key
-                                // z = kTcZ0 + 2^15 * hamming + column (tc_layout.cuh); 0 = the integer distance (XOR + POPC sweep)
-    int win_keys;               // row keys carry a WINDOW of train columns instead of a column (sweep_win.cu; see finalize.cu)
+    KeyFormat key_format;
     int phase;                  // 0 = everything in one launch; two-phase cross-check (finalize.cu): 1 = ratio test + list of the train rows to verify,
                                 // 2 = verdicts of the verification sweep + compaction
     int* gather;                // [n_pairs][stride] phase 1 out / the verification sweep's input

@@ -42,19 +42,17 @@ __device__ __forceinline__ void order2(float& da, int& ia, float& db, int& ib) {
     }
 }
 
-// Hamming distance out of the high word of a sweep key: the integer itself (XOR + POPC sweep), the float 2 * hamming (tensor-core
-// sweep), or the packed float key z = kTcZ0i + 2^15 * hamming + column (tensor-core sweep, "Z" encoding)
+// Hamming distance out of the high word of a sweep key (KeyFormat)
 __device__ __forceinline__ float b256_key_distance(const FinalizeParams& p, u64 k) {
     const uint32_t hi = (uint32_t)(k >> 32);
-    if (p.b256_float_keys == 2) return (float)(((int)__uint_as_float(hi) - kTcZ0i) >> kTcZShift);
-    if (p.b256_float_keys == 1) return 0.5f * __uint_as_float(hi);
-    return (float)hi;
+    if (p.key_format == KeyFormat::TcZ) return (float)(((int)__uint_as_float(hi) - kTcZ0i) >> kTcZShift);
+    if (p.key_format == KeyFormat::TcPm1) return 0.5f * __uint_as_float(hi);
+    return (float)hi;      // Direct (slice keys are read by eval_rows_win)
 }
 
 template <int KIND>
 __device__ __forceinline__ RowResult eval_row(const FinalizeParams& p, const u64* rk1, const u64* rk2, const u64* ck1,
-                                              const u64* ck2, const float* qrows, const float* trows, int q, int fq,
-                                              int32_t* knn_idx, float* knn_dist) {
+                                              const float* qrows, const float* trows, int q, int32_t* knn_idx, float* knn_dist) {
     RowResult r;
     r.keep = false;
     r.t1 = -1;
@@ -104,7 +102,6 @@ __device__ __forceinline__ RowResult eval_row(const FinalizeParams& p, const u64
     r.keep = true;
     r.t1 = i1;
     r.d1 = d1;
-    (void)fq;
     return r;
 }
 
@@ -346,7 +343,7 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
         if (p.phase == 1 && threadIdx.x == 0) p.gather_cnt[pair] = 0;
         if (p.knn_idx) {
             for (int q = threadIdx.x; q < fq; q += kFinThreads) {
-                RowResult r = eval_row<KIND>(p, rk1, rk2, ck1, ck2, qrows, trows, q, fq, p.knn_idx, p.knn_dist);     // (knn output: never slice keys)
+                RowResult r = eval_row<KIND>(p, rk1, rk2, ck1, qrows, trows, q, p.knn_idx, p.knn_dist);     // (knn output: never slice keys)
                 (void)r;
             }
         }
@@ -378,7 +375,7 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
         if (threadIdx.x == 0) s_targets = 0;
         __syncthreads();
     }
-    if (p.win_keys) {
+    if (p.key_format == KeyFormat::Slice) {
         const bool fast = KIND == ESFM_KIND_F32X64 && p.row_eps;
         const float* row_eps = fast ? p.row_eps + p.frame_row_off[pd.q_frame] : nullptr;
         const float nq = fast ? p.frame_norm[pd.q_frame] : 0.f, nt = fast ? p.frame_norm[pd.t_frame] : 0.f;
@@ -416,7 +413,7 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
         }
     } else {
     for (int q = threadIdx.x; q < fq; q += kFinThreads) {
-        const RowResult r = eval_row<KIND>(p, rk1, rk2, ck1, ck2, qrows, trows, q, fq, p.knn_idx, p.knn_dist);
+        const RowResult r = eval_row<KIND>(p, rk1, rk2, ck1, qrows, trows, q, p.knn_idx, p.knn_dist);
         rk1[q] = r.keep ? make_key(__float_as_uint(r.d1), (uint32_t)r.t1) : kKeyInit;
         mine += r.keep ? 1u : 0u;
     }

@@ -70,6 +70,11 @@ struct ChunkBuf {
 
 struct OrbState;                                 // scratch of the ORB extractor (orb.cu), kept between calls
 
+// The tensor-core operand image of a bank (tc_layout.cuh), built for the sweep that reads it.  SURF: the 3xTF32 hi / lo split (sweep_l2_tc.cu)
+// or the 16-bit "H" split (sweep_win.cu; followed by what win_fast_eps needs).  ORB: FP8 +-1 (sweep_l2_tc.cu's generic epilogue,
+// sweep_win.cu) or the FP8 "Z" encoding, whose accumulator is the packed key (sweep_l2_tc.cu).
+enum class TcImage { Tf32x3, H, Fp8Pm1, Fp8Z };
+
 }  // namespace esfm
 
 struct esfm_ctx {
@@ -89,8 +94,6 @@ struct esfm_ctx {
     esfm::u64* keys = nullptr;     size_t keys_bytes = 0;
     uint32_t* col_thr = nullptr;   size_t col_thr_elems = 0;
     int* gather_cnt = nullptr;     size_t gather_cnt_elems = 0;     // two-phase cross-check: train rows to verify, per pair of the chunk
-    int two_phase = 1;                     // cross-check of the tc16 sweeps as ratio test -> verification sweep over the surviving train rows
-                                           // ($ESFM_TWO_PHASE=0: column minima inside the one sweep, as the other engines do)
     int tc16_exact = 0;                    // $ESFM_TC16_EXACT=1: SURF tc16 sweeps in exact mode (13 MMA slots per tile) instead of fast mode
                                            // (9 slots) + exact fallback sweep of the rows it cannot settle
     esfm::ChunkBuf buf[2];
@@ -131,7 +134,7 @@ struct esfm_bank {
     bool kmajor_built = false;
     unsigned char* d_tc = nullptr; size_t tc_bytes = 0; size_t tc_cap = 0;       // tensor-core operand images, built on first use
     bool tc_built = false;
-    int tc_z = 0;                                         // ... of a B256 bank: 0 = +-1 encoding, 1 = "Z" encoding (tc_layout.cuh)
+    esfm::TcImage tc_image = esfm::TcImage::Tf32x3;       // ... which one
     int* d_tables = nullptr;                              // frame_rows | row_off | tile_off, (n_frames + 1) ints each
     int* d_frame_rows = nullptr;
     int* d_row_off = nullptr;

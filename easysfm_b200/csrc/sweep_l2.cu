@@ -64,7 +64,6 @@ __device__ __forceinline__ UnitInfo decode_unit(const SweepParams& p, int unit) 
 }  // namespace
 
 constexpr int kScratchStride = 20;          // floats per lane (16 used; 80-byte stride keeps STS.128 conflict-free)
-constexpr uint32_t kThrInit = 0x7f7f7f7fu;  // 3.39e38f: what a byte-wise memset(0x7f) of the threshold arrays produces
 constexpr int kStageFloats = kTileFloats + kTile;   // tile + the 128 column thresholds that travel with it
 constexpr int kStageBytes = kStageFloats * 4;
 

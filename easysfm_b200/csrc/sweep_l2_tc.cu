@@ -12,19 +12,20 @@
 // whose accumulator is the packed key 20480 + 2^15 hamming + column: branch-free row selection; the default).
 //
 // One persistent CTA per SM, 24 warps, four pipelines (TMA -> shared memory -> tensor memory -> registers).  A CTA works
-// on a QUERY BLOCK of QT (template parameter, 1 or 2) 128-row tiles at a time and streams the train frame past it once.
+// on one 128-row QUERY TILE at a time and streams the train frame past it once.  (A variant with two query tiles per block,
+// every train tile feeding two accumulators, measured slower in round 1 and was removed.)
 //   warp 16 (one lane)  TMA producer: one cp.async.bulk per 128-row train tile image (SURF 68 KB, ORB 36 KB: main + augmented
 //                       columns) into a 3-stage full/empty mbarrier ring; the 128 running column thresholds of the tile ride
 //                       in their own 4-stage ring.
-//   warp 17             MMA issuer (warp-uniform control flow, one elected lane issues): per (train tile, query tile)
+//   warp 17             MMA issuer (warp-uniform control flow, one elected lane issues): per train tile
 //                       SURF: 25 x tcgen05.mma.cta_group::1.kind::tf32 (M=128, N=128, K=8) = 3 terms (lo.hi, hi.lo, hi.hi) x 8
 //                       k-steps + 1 augmented k-step that adds both half norms exactly; ORB: 8 + 1 x kind::f8f6f4 (K=32).
 //                       The query operand is read from TENSOR MEMORY, the train operand from SWIZZLE_128B shared-memory atoms;
-//                       the result accumulates in one of the tensor-memory stages (128 columns each: 3 stages at QT = 1);
+//                       the result accumulates in one of the 3 tensor-memory stages (128 columns each);
 //                       tcgen05.commit publishes the accumulator stage and releases the shared-memory stage.
-//   warps 20-23         query writers: rows of query tile h -> operand columns of tensor memory (tcgen05.st; SURF: fp32 ->
+//   warps 20-23         query writers: rows of the query tile -> operand columns of tensor memory (tcgen05.st; SURF: fp32 ->
 //                       (hi, lo) TF32, ORB: bits -> FP8) + the tile's augmented block in shared memory; they block on a
-//                       named barrier until the epilogue has seen the last accumulator that read the slot.
+//                       named barrier until the epilogue has seen the last accumulator that read the previous tile.
 //   warps 0-15          epilogue: warp w owns TMEM lanes 32*(w%4).. (= query rows) and column quarter w/4.  tcgen05.ld
 //                       gives each THREAD one query row x 32 train columns, so the row's running top-2 is thread-private
 //                       (no shuffles); column minima go through a warp REDUX + one fire-and-forget atomicMin per hit.
@@ -35,49 +36,37 @@ namespace esfm {
 
 namespace {
 
-// Geometry variants (template parameter QT = query tiles per block): tensor memory has 512 columns = QT x 128 of query
-// operand (hi 64 | lo 64 per tile) + the accumulator stages (128 columns each).
-//   QT = 1: 3 accumulator stages; every train tile in shared memory feeds one accumulator.
-//   QT = 2: 2 accumulator stages; every train tile feeds two accumulators (half the L2 -> shared-memory traffic and power).
+// Tensor memory has 512 columns: the query operand (SURF hi 64 | lo 64 = 128 columns, ORB 64) + the accumulator stages (128 columns
+// each), 3 stages for both kinds.
+constexpr int kTcAccStages = 3;
+constexpr uint32_t kTcACol0 = 128u * kTcAccStages;     // tensor-memory column of the query operand
+static_assert(kTcACol0 + 128 <= 512, "tensor memory: accumulator stages + SURF query operand");
+}  // namespace
+
 // KIND = ESFM_KIND_F32X64: 3xTF32, query operand = 128 columns (hi 64 | lo 64), train tile image 68 KB;
 // KIND = ESFM_KIND_B256:   Hamming as an FP8 +-1 dot product (tc_layout.cuh), query operand = 64 columns, image 36 KB.
 // KIND = kTcKindB256Z:     the same with scaled operands whose accumulator is the packed key z = Z0 + 2^15 hamming + column
-//                          (tc_layout.cuh "Z" encoding): branch-free row selection, QT = 1 only.
-template <int QT, int KIND> struct TcGeom {
-    static constexpr int kACols = tc_kind_is_f32(KIND) ? 128 : 64;
-    static constexpr int kAccStages = (512 - QT * kACols) / 128;
-    static constexpr uint32_t kACol0 = 128u * kAccStages;   // tensor-memory column of query tile 0's operand
-    static constexpr int kMainBytes = tc_kind_is_f32(KIND) ? kTcMainBytes : kTc8MainBytes;
-    static constexpr int kGroupBytes = tc_kind_is_f32(KIND) ? kTcGroupBytes : kTc8GroupBytes;
-    static constexpr int kTileBytes = kMainBytes + kTcAugBytes;
-};
-}  // namespace
-
-template <int kTcQTiles, int KIND>
+//                          (tc_layout.cuh "Z" encoding): branch-free row selection.
+template <int KIND>
 __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepParams p) {
-    using G = TcGeom<kTcQTiles, KIND>;
-    constexpr int kTcAccStages = G::kAccStages;
-    constexpr uint32_t kTcACol0 = G::kACol0;
-    constexpr int kACols = G::kACols;
-    constexpr int kTcTileBytes = G::kTileBytes;       // (shadows the SURF constant of tc_layout.cuh)
-    constexpr int kTcMainBytes = G::kMainBytes;
-    constexpr int kTcGroupBytes = G::kGroupBytes;
-    constexpr uint32_t kTcBoundBits = tc_kind_is_f32(KIND) ? kTcBoundBitsF32 : (KIND == kTcKindB256Z ? kTcBoundBitsZ : kTcBoundBitsB256);
     constexpr bool kOrb = !tc_kind_is_f32(KIND);          // FP8 operands (both ORB encodings share the MMA sequence and the tile geometry)
     constexpr bool kZ = KIND == kTcKindB256Z;
-    static_assert(!kZ || kTcQTiles == 1, "the Z epilogue keeps one row state per thread");
+    constexpr int kTcMainBytes = kOrb ? kTc8MainBytes : esfm::kTcMainBytes;
+    constexpr int kTcGroupBytes = kOrb ? kTc8GroupBytes : esfm::kTcGroupBytes;
+    constexpr int kTcTileBytes = kTcMainBytes + kTcAugBytes;     // (shadows the SURF constant of tc_layout.cuh)
+    constexpr uint32_t kTcBoundBits = tc_kind_is_f32(KIND) ? kTcBoundBitsF32 : (kZ ? kTcBoundBitsZ : kTcBoundBitsB256);
     extern __shared__ unsigned char smem_raw[];
     // SWIZZLE_128B atoms need 1024-byte alignment
     unsigned char* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
     unsigned char* Ts = base;                                   // kTcStages train tile images (each 68 x 1024 B: atoms stay aligned)
-    unsigned char* Qa = Ts + kTcStages * kTcTileBytes;          // augmented blocks (1, 1, 1, hq_h | hq_m, hq_l, 0, 0) of the two query tiles
-    unsigned char* Thr = Qa + kTcQTiles * kTcAugBytes;          // kTcThrStages x 128 column thresholds
-    u64* mkey = reinterpret_cast<u64*>(Thr + kTcThrStages * kTcThrBytes);          // [tile h][best, second][128] merged row keys
-    uint32_t* sbound = reinterpret_cast<uint32_t*>(mkey + kTcQTiles * 2 * kTile);  // [tile h][128] row bound shared by a row's parts
-    float* colsc = reinterpret_cast<float*>(sbound + kTcQTiles * kTile);          // [epilogue warp][4 columns][32 lanes] column-event scratch
+    unsigned char* Qa = Ts + kTcStages * kTcTileBytes;          // augmented block (1, 1, 1, hq_h | hq_m, hq_l, 0, 0) of the query tile
+    unsigned char* Thr = Qa + kTcAugBytes;                      // kTcThrStages x 128 column thresholds
+    u64* mkey = reinterpret_cast<u64*>(Thr + kTcThrStages * kTcThrBytes);          // [best, second][128] merged row keys
+    uint32_t* sbound = reinterpret_cast<uint32_t*>(mkey + 2 * kTile);             // [128] row bound shared by a row's parts
+    float* colsc = reinterpret_cast<float*>(sbound + kTile);                      // [epilogue warp][4 columns][32 lanes] column-event scratch
     uint64_t* bars = reinterpret_cast<uint64_t*>(reinterpret_cast<unsigned char*>(colsc) + kTcScBytes);
-    uint64_t* fullQ = bars;                      // [kTcQTiles]
-    uint64_t* fullT = fullQ + kTcQTiles;
+    uint64_t* fullQ = bars;
+    uint64_t* fullT = fullQ + 1;
     uint64_t* emptyT = fullT + kTcStages;
     uint64_t* accFull = emptyT + kTcStages;
     uint64_t* accEmpty = accFull + kTcAccStages;
@@ -89,9 +78,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
     const int n_units = p.n_pairs * p.units_per_pair;
 
     if (threadIdx.x == 0) {
-        for (int h = 0; h < kTcQTiles; ++h) {
-            mbar_init(&fullQ[h], 4);                  // the 4 query-writer warps
-        }
+        mbar_init(fullQ, 4);                          // the 4 query-writer warps
         for (int s = 0; s < kTcStages; ++s) {
             mbar_init(&fullT[s], 1);
             mbar_init(&emptyT[s], 1);                 // MMA commit
@@ -122,7 +109,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                 const TcUnit u = tc_decode_unit(p, unit);
                 const unsigned char* timg = p.tc_main + (size_t)p.frame_tile_off[u.t_frame] * kTcTileBytes;
                 const uint32_t* tauc = p.col_thr + (size_t)u.pair * p.stride;
-                for (int qt = u.qb0; qt < u.qb1; qt += kTcQTiles) {
+                for (int qt = u.qb0; qt < u.qb1; ++qt) {
                     for (int tt = 0; tt < u.ntt; ++tt, ++g) {
                         const uint32_t st = g % kTcStages, ph = (g / kTcStages) & 1;
                         mbar_wait_sleep<kTcSleepProducer>(&emptyT[st], ph ^ 1);
@@ -151,67 +138,61 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
         const uint64_t qad0 = tc_desc_nosw(smem_u32(Qa), 128, kTcAugGroupBytes);
         const uint64_t td0 = tc_desc_sw128(smem_u32(Ts), kTcGroupBytes);
         const uint64_t tad0 = tc_desc_nosw(smem_u32(Ts) + kTcMainBytes, 128, kTcAugGroupBytes);
-        uint32_t g = 0, a = 0;               // train tiles streamed, accumulator jobs issued
-        uint32_t qn0 = 0, qn1 = 0;           // how many times query slot 0 / 1 has been filled (slot 1 is absent from an odd tail block)
+        const uint32_t acol = tmem + kTcACol0;
+        uint32_t g = 0;                      // train tiles streamed = accumulator jobs issued
+        uint32_t qn = 0;                     // how many times the query operand has been filled
         for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
             const TcUnit u = tc_decode_unit(p, unit);
-            for (int qt = u.qb0; qt < u.qb1; qt += kTcQTiles) {
-                const int nh = min(kTcQTiles, u.qb1 - qt);
+            for (int qt = u.qb0; qt < u.qb1; ++qt, ++qn) {
                 for (int tt = 0; tt < u.ntt; ++tt, ++g) {
                     const uint32_t st = g % kTcStages, ph = (g / kTcStages) & 1;
                     mbar_wait_sleep<kTcSleepIssuer>(&fullT[st], ph);
                     // descriptor start addresses are in 16-byte units: adding (bytes >> 4) to the low word moves the window
                     const uint64_t td = td0 + (uint64_t)(st * (kTcTileBytes >> 4));
                     const uint64_t tad = tad0 + (uint64_t)(st * (kTcTileBytes >> 4));
-#pragma unroll 1
-                    for (int h = 0; h < nh; ++h, ++a) {
-                        const uint32_t as = a % kTcAccStages, aph = (a / kTcAccStages) & 1;
-                        if (tt == 0) mbar_wait_sleep<kTcSleepIssuer>(&fullQ[h], (h == 0 ? qn0 : qn1) & 1);   // the writers have filled slot h for this block
-                        mbar_wait_sleep<kTcSleepIssuer>(&accEmpty[as], aph ^ 1);
-                        tc_fence_after();
-                        const uint32_t d = tmem + as * 128;
-                        const uint32_t acol = tmem + kTcACol0 + h * kACols;
-                        if (kOrb) {
-                            if (!(p.debug_flags & 2) && elect_one()) {
-                                // 256 FP8 values per row = 8 k-steps of K = 32 (32 bytes: the same descriptor arithmetic as TF32's K = 8)
-#pragma unroll
-                                for (int ks = 0; ks < 8; ++ks) {
-                                    const uint32_t off = ((ks >> 2) * 1024 + (ks & 3) * 32) >> 4;
-                                    tc_mma_f8_ts(d, acol + ks * 8, td + (uint64_t)off, idesc, ks > 0);
-                                }
-                                // - 256 and the pad-row penalties (tc_layout.cuh)
-                                tc_mma_f8(d, qad0 + (uint64_t)(h * (kTcAugBytes >> 4)), tad, idesc, true);
-                            }
-                        } else
+                    const uint32_t as = g % kTcAccStages, aph = (g / kTcAccStages) & 1;
+                    if (tt == 0) mbar_wait_sleep<kTcSleepIssuer>(fullQ, qn & 1);   // the writers have filled the query operand for this tile
+                    mbar_wait_sleep<kTcSleepIssuer>(&accEmpty[as], aph ^ 1);
+                    tc_fence_after();
+                    const uint32_t d = tmem + as * 128;
+                    if (kOrb) {
                         if (!(p.debug_flags & 2) && elect_one()) {
-                            bool first = true;
+                            // 256 FP8 values per row = 8 k-steps of K = 32 (32 bytes: the same descriptor arithmetic as TF32's K = 8)
 #pragma unroll
-                            for (int term = 0; term < 3; ++term) {
-                                // (A part, B part): lo.hi, hi.lo first (small terms), hi.hi last
-                                const int pa = term == 0 ? 1 : 0, pb = term == 1 ? 1 : 0;
-#pragma unroll
-                                for (int ks = 0; ks < 8; ++ks) {
-                                    const uint32_t off = ((ks >> 2) * 1024 + (ks & 3) * 32) >> 4;
-                                    // A (query) from tensor memory: lane = row, column = k.  With both operands in shared memory the
-                                    // 8 KB of operand reads per MMA plus the TMA writes saturate the 128 B/clk shared-memory port
-                                    // (measured 87 cycles per MMA instead of 64).
-                                    tc_mma_tf32_ts(d, acol + pa * 64 + ks * 8, td + (uint64_t)(pb * (2048 >> 4) + off), idesc, !first);
-                                    first = false;
-                                }
+                            for (int ks = 0; ks < 8; ++ks) {
+                                const uint32_t off = ((ks >> 2) * 1024 + (ks & 3) * 32) >> 4;
+                                tc_mma_f8_ts(d, acol + ks * 8, td + (uint64_t)off, idesc, ks > 0);
                             }
-                            // - 1/2|q|^2 - 1/2|t|^2, exact (three-way split half norms against ones)
-                            tc_mma_tf32(d, qad0 + (uint64_t)(h * (kTcAugBytes >> 4)), tad, idesc, true);
+                            // - 256 and the pad-row penalties (tc_layout.cuh)
+                            tc_mma_f8(d, qad0, tad, idesc, true);
                         }
-                        __syncwarp();
-                        if (elect_one()) {
-                            tc_commit(&accFull[as]);                        // accumulator stage ready for the epilogue
-                            if (h == nh - 1) tc_commit(&emptyT[st]);        // shared-memory stage consumed
+                    } else
+                    if (!(p.debug_flags & 2) && elect_one()) {
+                        bool first = true;
+#pragma unroll
+                        for (int term = 0; term < 3; ++term) {
+                            // (A part, B part): lo.hi, hi.lo first (small terms), hi.hi last
+                            const int pa = term == 0 ? 1 : 0, pb = term == 1 ? 1 : 0;
+#pragma unroll
+                            for (int ks = 0; ks < 8; ++ks) {
+                                const uint32_t off = ((ks >> 2) * 1024 + (ks & 3) * 32) >> 4;
+                                // A (query) from tensor memory: lane = row, column = k.  With both operands in shared memory the
+                                // 8 KB of operand reads per MMA plus the TMA writes saturate the 128 B/clk shared-memory port
+                                // (measured 87 cycles per MMA instead of 64).
+                                tc_mma_tf32_ts(d, acol + pa * 64 + ks * 8, td + (uint64_t)(pb * (2048 >> 4) + off), idesc, !first);
+                                first = false;
+                            }
                         }
-                        __syncwarp();
+                        // - 1/2|q|^2 - 1/2|t|^2, exact (three-way split half norms against ones)
+                        tc_mma_tf32(d, qad0, tad, idesc, true);
                     }
+                    __syncwarp();
+                    if (elect_one()) {
+                        tc_commit(&accFull[as]);                        // accumulator stage ready for the epilogue
+                        tc_commit(&emptyT[st]);                         // shared-memory stage consumed
+                    }
+                    __syncwarp();
                 }
-                ++qn0;
-                if (nh == kTcQTiles) ++qn1;
             }
         }
     } else if (warp >= kTcWriterWarp0) {
@@ -219,7 +200,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
         const int quarter = warp & 3;
         const int trow = quarter * 32 + lane;
         const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
-        uint32_t quse[2] = {0, 0};
+        bool filled = false;                // the query operand has been filled before: wait until the epilogue is done with it
         for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
             const TcUnit u = tc_decode_unit(p, unit);
             const int fq = p.frame_rows[u.q_frame];
@@ -227,17 +208,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                 // ---- ORB: 256 bits -> 256 FP8 values +-1.0 (Z encoding: +-256), 4 per tensor-memory column ----
                 const uint4* qbits = p.rows_b256 + (size_t)p.frame_row_off[u.q_frame] * 2;
                 for (int qt = u.qb0; qt < u.qb1; ++qt) {
-                    const int h = (qt - u.qb0) & (kTcQTiles - 1);
                     const int r = qt * kTile + trow;
                     const bool valid = r < fq;
                     uint4 w0 = make_uint4(0u, 0u, 0u, 0u), w1 = w0;
                     if (valid) { w0 = __ldg(qbits + (size_t)r * 2); w1 = __ldg(qbits + (size_t)r * 2 + 1); }
-                    const uint32_t use = h == 0 ? quse[0] : quse[1];
-                    if (use > 0) named_bar_sync(2 + h, 128 + 32);      // slot h free (see the SURF branch below)
-                    if (h == 0) ++quse[0]; else ++quse[1];
+                    if (filled) named_bar_sync(2, 128 + 32);      // operand free (see the SURF branch below)
+                    filled = true;
                     tc_fence_after();
                     // augmented columns: (qpad ? 448 : 0, 448, 16, 0 ...) in FP8; Z encoding: the offset slots and digit multipliers
-                    unsigned char* qa = Qa + h * kTcAugBytes + (trow >> 3) * kTcAugGroupBytes + (trow & 7) * 16;
+                    unsigned char* qa = Qa + (trow >> 3) * kTcAugGroupBytes + (trow & 7) * 16;
                     if (kZ) {
                         uint32_t aw[8];
                         tcz_query_aug(aw);
@@ -248,7 +227,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                         *reinterpret_cast<uint4*>(qa + 128) = make_uint4(0u, 0u, 0u, 0u);
                     }
                     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    const uint32_t acol = tmem + lane_addr + kTcACol0 + h * kACols;
+                    const uint32_t acol = tmem + lane_addr + kTcACol0;
                     const uint32_t ws[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
 #pragma unroll
                     for (int m = 0; m < 8; ++m) {       // word m = elements 32 m .. 32 m + 31 = 8 columns
@@ -260,13 +239,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                     tmem_st_wait();
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) mbar_arrive(&fullQ[h]);
+                    if (lane == 0) mbar_arrive(fullQ);
                 }
                 continue;
             }
             const float4* qrows = reinterpret_cast<const float4*>(p.rows_f32 + (size_t)p.frame_row_off[u.q_frame] * kDim);
             for (int qt = u.qb0; qt < u.qb1; ++qt) {
-                const int h = (qt - u.qb0) & (kTcQTiles - 1);
                 const int r = qt * kTile + trow;
                 const bool valid = r < fq;
                 const float4* xr = qrows + (size_t)(valid ? r : 0) * 16;
@@ -281,19 +259,18 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                 float hq = valid ? 0.5f * hs : kTcPadNorm;   // pad rows can never win a column
                 float hqh, hqm, hql;
                 tc_split3(hq, hqh, hqm, hql);
-                const uint32_t use = h == 0 ? quse[0] : quse[1];
-                // Slot h is free once every MMA that read its previous tile has retired.  The writers do not poll for that (four
-                // warps polling an mbarrier for a whole query block were 20 % of all executed instructions; __nanosleep does not
-                // sleep anywhere near the requested time): they block on NAMED BARRIER 2 + h, which epilogue warp 0 arrives at
-                // as soon as it has seen the accumulator of the block's last (train tile, slot h) job complete.
-                if (use > 0) named_bar_sync(2 + h, 128 + 32);
-                if (h == 0) ++quse[0]; else ++quse[1];
+                // The operand is free once every MMA that read the previous query tile has retired.  The writers do not poll for
+                // that (four warps polling an mbarrier for a whole query tile were 20 % of all executed instructions; __nanosleep does
+                // not sleep anywhere near the requested time): they block on NAMED BARRIER 2, which epilogue warp 0 arrives at as
+                // soon as it has seen the accumulator of the previous tile's last train tile complete.
+                if (filled) named_bar_sync(2, 128 + 32);
+                filled = true;
                 tc_fence_after();
-                unsigned char* qa = Qa + h * kTcAugBytes + (trow >> 3) * kTcAugGroupBytes + (trow & 7) * 16;
+                unsigned char* qa = Qa + (trow >> 3) * kTcAugGroupBytes + (trow & 7) * 16;
                 *reinterpret_cast<float4*>(qa) = make_float4(1.f, 1.f, 1.f, hqh);
                 *reinterpret_cast<float4*>(qa + 128) = make_float4(hqm, hql, 0.f, 0.f);
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy stores -> visible to the MMA's async reads
-                const uint32_t acol = tmem + lane_addr + kTcACol0 + h * kACols;
+                const uint32_t acol = tmem + lane_addr + kTcACol0;
                 // pass 2: the row again (L1/L2 hit), 8 dims at a time -> hi / lo columns of tensor memory
 #pragma unroll 2
                 for (int m = 0; m < 8; ++m) {
@@ -313,12 +290,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                 tmem_st_wait();
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) mbar_arrive(&fullQ[h]);
+                if (lane == 0) mbar_arrive(fullQ);
             }
         }
-        // the epilogue arrives once per (block, slot); the last arrival of each slot has no refill waiting for it
-        if (quse[0] > 0) named_bar_sync(2, 128 + 32);
-        if (kTcQTiles == 2 && quse[1] > 0) named_bar_sync(3, 128 + 32);
+        // the epilogue arrives once per query tile; the last arrival has no refill waiting for it
+        if (filled) named_bar_sync(2, 128 + 32);
     }
     } else {
         // ======================= epilogue warps =======================
@@ -326,21 +302,20 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
         const int quarter = warp & 3, part = warp >> 2;
         const int trow = quarter * 32 + lane;               // row inside a 128-row query tile (= TMEM lane)
         const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
-        if (part < kTcQTiles) {
-            sbound[part * kTile + trow] = kTcBoundBits;
-            mkey[(part * 2) * kTile + trow] = kKeyInit;
-            mkey[(part * 2 + 1) * kTile + trow] = kKeyInit;
+        if (part == 0) {
+            sbound[trow] = kTcBoundBits;
+            mkey[trow] = kKeyInit;
+            mkey[kTile + trow] = kKeyInit;
         }
         asm volatile("bar.sync 1, %0;" ::"n"(kTcEpiThreads) : "memory");
-        uint32_t g = 0, a = 0;
+        uint32_t g = 0;                     // train tiles seen = accumulators read
         for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
             const TcUnit u = tc_decode_unit(p, unit);
             u64* rk1 = p.keys + (size_t)u.pair * 4 * p.stride;
             u64* rk2 = rk1 + p.stride;
             u64* ck1 = rk2 + p.stride;
             uint32_t* tauc = p.col_thr + (size_t)u.pair * p.stride;
-            for (int qt = u.qb0; qt < u.qb1; qt += kTcQTiles) {
-                const int nh = min(kTcQTiles, u.qb1 - qt);
+            for (int qt = u.qb0; qt < u.qb1; ++qt) {
                 if constexpr (kZ) {
                     // ================= ORB, "Z" encoding: the accumulator IS the packed key z = Z0 + 2^15 hamming + column =================
                     // Every element of a row is a distinct positive integer-valued float, smaller = nearer, ties = lower column, so the
@@ -355,13 +330,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                     // several CTAs other CTAs' (higher) rows are in the snapshot too and equal distances must still get through.
                     const float thr_sub = p.units_per_pair == 1 ? 1.f : 0.f;
                     float k1 = kTcZNone, k2 = kTcZNone;
-                    for (int tt = 0; tt < u.ntt; ++tt, ++g, ++a) {
+                    for (int tt = 0; tt < u.ntt; ++tt, ++g) {
                         const uint32_t ts = g % kTcThrStages, tph = (g / kTcThrStages) & 1;
                         mbar_wait_sleep<kTcSleepEpilogue>(&thrFull[ts], tph);
                         const float4* tp = reinterpret_cast<const float4*>(Thr + ts * kTcThrBytes) + part * (kTcPartCols / 4);
-                        const uint32_t as = a % kTcAccStages, aph = (a / kTcAccStages) & 1;
+                        const uint32_t as = g % kTcAccStages, aph = (g / kTcAccStages) & 1;
                         mbar_wait_sleep<kTcSleepEpilogue>(&accFull[as], aph);
-                        if (warp == 0 && tt == u.ntt - 1) named_bar_arrive(2, 128 + 32);     // the query slot may be refilled (see the writers)
+                        if (warp == 0 && tt == u.ntt - 1) named_bar_arrive(2, 128 + 32);     // the query operand may be refilled (see the writers)
                         tc_fence_after();
                         uint32_t vb[32];
                         tmem_ld32(tmem + lane_addr + as * 128 + part * kTcPartCols, vb);
@@ -459,34 +434,32 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                         }
                     }
                 } else {
-                    // running top-2 of this thread's row in query tile 0 (t) and tile 1 (to); the two swap after every accumulator
-                    RowTop2 t, to;
-                    t.v1 = t.v2 = to.v1 = to.v2 = __uint_as_float(kTcBoundBits);
-                    t.i1 = t.i2 = to.i1 = to.i2 = 0xffffffffu;
+                    // running top-2 of this thread's row
+                    RowTop2 t;
+                    t.v1 = t.v2 = __uint_as_float(kTcBoundBits);
+                    t.i1 = t.i2 = 0xffffffffu;
+                    const uint32_t qrow = (uint32_t)(qt * kTile + trow);     // frame row of this thread
+                    uint32_t* sb = &sbound[trow];
                     for (int tt = 0; tt < u.ntt; ++tt, ++g) {
                         const uint32_t ts = g % kTcThrStages, tph = (g / kTcThrStages) & 1;
                         mbar_wait_sleep<kTcSleepEpilogue>(&thrFull[ts], tph);
                         const float4* tp = reinterpret_cast<const float4*>(Thr + ts * kTcThrBytes) + part * (kTcPartCols / 4);
-    #pragma unroll 1
-                        for (int h = 0; h < nh; ++h, ++a) {
-                            const uint32_t as = a % kTcAccStages, aph = (a / kTcAccStages) & 1;
-                            const uint32_t qrow = (uint32_t)((qt + h) * kTile + trow);     // frame row of this thread
-                            uint32_t* sb = &sbound[h * kTile + trow];
-                            mbar_wait_sleep<kTcSleepEpilogue>(&accFull[as], aph);
-                            if (warp == 0 && tt == u.ntt - 1) named_bar_arrive(2 + h, 128 + 32);   // slot h may be refilled (see the writers)
-                            tc_fence_after();
-                            // All 32 columns of this thread go to registers at once and the accumulator stage is released right
-                            // away: the tensor pipe never waits for the selection logic below.
-                            uint32_t vb[32];
-                            tmem_ld32(tmem + lane_addr + as * 128 + part * kTcPartCols, vb);
-                            // The row's running second best over ALL column parts (each part keeps a private top-2; the shared
-                            // bound only filters, with '>=' so equal values still reach the private strict-'<' insertion).
-                            float nb = -__uint_as_float(*reinterpret_cast<volatile uint32_t*>(sb));
-                            tmem_ld_wait();
-                            tc_fence_before();
-                            __syncwarp();
-                            if (lane == 0) mbar_arrive_relaxed(&accEmpty[as]);
-                            if (p.debug_flags & 1) continue;
+                        const uint32_t as = g % kTcAccStages, aph = (g / kTcAccStages) & 1;
+                        mbar_wait_sleep<kTcSleepEpilogue>(&accFull[as], aph);
+                        if (warp == 0 && tt == u.ntt - 1) named_bar_arrive(2, 128 + 32);   // the query operand may be refilled (see the writers)
+                        tc_fence_after();
+                        // All 32 columns of this thread go to registers at once and the accumulator stage is released right
+                        // away: the tensor pipe never waits for the selection logic below.
+                        uint32_t vb[32];
+                        tmem_ld32(tmem + lane_addr + as * 128 + part * kTcPartCols, vb);
+                        // The row's running second best over ALL column parts (each part keeps a private top-2; the shared
+                        // bound only filters, with '>=' so equal values still reach the private strict-'<' insertion).
+                        float nb = -__uint_as_float(*reinterpret_cast<volatile uint32_t*>(sb));
+                        tmem_ld_wait();
+                        tc_fence_before();
+                        __syncwarp();
+                        if (lane == 0) mbar_arrive_relaxed(&accEmpty[as]);
+                        if (!(p.debug_flags & 1)) {
                             float v[32];
     #pragma unroll
                             for (int c = 0; c < 32; ++c) v[c] = __uint_as_float(vb[c]);   // v = -1/2 d^2
@@ -582,43 +555,31 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
                                     if (ins) atomicMin(sb, __float_as_uint(fmaxf(t.v2, 0.f)));
                                 }
                             }
-                            if (kTcQTiles == 2 && nh == 2) {      // next accumulator belongs to the other query tile
-                                const RowTop2 x = t;
-                                t = to;
-                                to = x;
-                            }
                         }
                         __syncwarp();
                         if (lane == 0) mbar_arrive_relaxed(&thrEmpty[ts]);      // last read of this threshold snapshot
                     }
                     // ---- end of the sweep for this query block: merge the column parts of every row, publish ----
-                    // 64-bit shared-memory atomics on packed keys: the smallest key ends in mkey[.][0], the smallest of all the
-                    // "losers" (displaced old minimum, or the newcomer if it did not win) in mkey[.][1] = the second smallest overall.
-                    // (an even number of swaps per train tile: t is tile 0's state again, `to` tile 1's)
+                    // 64-bit shared-memory atomics on packed keys: the smallest key ends in mkey[0][.], the smallest of all the
+                    // "losers" (displaced old minimum, or the newcomer if it did not win) in mkey[1][.] = the second smallest overall.
     #pragma unroll
-                    for (int h = 0; h < kTcQTiles; ++h) {
-                        if (h < nh) {
-    #pragma unroll
-                            for (int e = 0; e < 2; ++e) {
-                                const RowTop2& s = h ? to : t;
-                                const uint32_t idx = e ? s.i2 : s.i1;
-                                if (idx != 0xffffffffu) {
-                                    const u64 k = make_key(__float_as_uint(fmaxf(e ? s.v2 : s.v1, 0.f)), idx);
-                                    const u64 old = atomicMin(&mkey[(h * 2) * kTile + trow], k);
-                                    atomicMin(&mkey[(h * 2 + 1) * kTile + trow], old > k ? old : k);
-                                }
-                            }
+                    for (int e = 0; e < 2; ++e) {
+                        const uint32_t idx = e ? t.i2 : t.i1;
+                        if (idx != 0xffffffffu) {
+                            const u64 k = make_key(__float_as_uint(fmaxf(e ? t.v2 : t.v1, 0.f)), idx);
+                            const u64 old = atomicMin(&mkey[trow], k);
+                            atomicMin(&mkey[kTile + trow], old > k ? old : k);
                         }
                     }
                 }   // (generic epilogue)
                 asm volatile("bar.sync 1, %0;" ::"n"(kTcEpiThreads) : "memory");
-                if (part < nh) {       // column part h publishes (and resets) query tile h
-                    const uint32_t qrow = (uint32_t)((qt + part) * kTile + trow);
-                    rk1[qrow] = mkey[(part * 2) * kTile + trow];
-                    rk2[qrow] = mkey[(part * 2 + 1) * kTile + trow];
-                    mkey[(part * 2) * kTile + trow] = kKeyInit;
-                    mkey[(part * 2 + 1) * kTile + trow] = kKeyInit;
-                    sbound[part * kTile + trow] = kTcBoundBits;
+                if (part == 0) {       // column part 0 publishes (and resets) the query tile
+                    const uint32_t qrow = (uint32_t)(qt * kTile + trow);
+                    rk1[qrow] = mkey[trow];
+                    rk2[qrow] = mkey[kTile + trow];
+                    mkey[trow] = kKeyInit;
+                    mkey[kTile + trow] = kKeyInit;
+                    sbound[trow] = kTcBoundBits;
                 }
                 asm volatile("bar.sync 1, %0;" ::"n"(kTcEpiThreads) : "memory");   // mkey[] / sbound[] are reused by the next query block
             }
@@ -631,12 +592,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) sweep_l2_tc_kernel(const SweepP
     if (warp == kTcEpiWarps + 1) tmem_free(tmem, 512);
 }
 
-size_t sweep_tc_smem_bytes(int qt, int kind) {
+size_t sweep_tc_smem_bytes(int kind) {
     const size_t tile = tc_kind_is_f32(kind) ? (size_t)kTcTileBytes : (size_t)kTc8TileBytes;
-    const int acc = (512 - qt * (tc_kind_is_f32(kind) ? 128 : 64)) / 128;
-    return 1024 + (size_t)kTcStages * tile + (size_t)qt * kTcAugBytes + (size_t)kTcThrStages * kTcThrBytes +
-           (size_t)qt * 2 * kTile * sizeof(u64) + (size_t)qt * kTile * 4 + (size_t)kTcScBytes +
-           (qt + 2 * kTcStages + 2 * acc + 2 * kTcThrStages) * 8 + 16;
+    return 1024 + (size_t)kTcStages * tile + (size_t)kTcAugBytes + (size_t)kTcThrStages * kTcThrBytes +
+           (size_t)2 * kTile * sizeof(u64) + (size_t)kTile * 4 + (size_t)kTcScBytes +
+           (1 + 2 * kTcStages + 2 * kTcAccStages + 2 * kTcThrStages) * 8 + 16;
 }
 
 // kind = p.tc_kind: ESFM_KIND_F32X64 (3xTF32 L2 sweep) or ESFM_KIND_B256 (FP8 Hamming sweep)
@@ -645,12 +605,10 @@ cudaError_t launch_sweep_l2_tc(const SweepParams& p, int sm_count, cudaStream_t 
     if (n_units <= 0) return cudaSuccess;
     const int grid = n_units < sm_count ? n_units : sm_count;
     const int kind = p.tc_kind == kTcKindB256Z ? p.tc_kind : (p.tc_kind == ESFM_KIND_B256 ? ESFM_KIND_B256 : ESFM_KIND_F32X64);
-    const int qt = 1;      // (two query tiles per block, $ESFM_TC_QT=2 in round 1: measured slower, and its shared memory has no room
-                           //  for the column-event scratch; the template parameter stays, the instantiations are gone)
-    const size_t smem = sweep_tc_smem_bytes(qt, kind);
+    const size_t smem = sweep_tc_smem_bytes(kind);
     void (*kern)(const SweepParams) =
-        kind == kTcKindB256Z ? sweep_l2_tc_kernel<1, kTcKindB256Z>
-        : kind == ESFM_KIND_B256 ? sweep_l2_tc_kernel<1, ESFM_KIND_B256> : sweep_l2_tc_kernel<1, ESFM_KIND_F32X64>;
+        kind == kTcKindB256Z ? sweep_l2_tc_kernel<kTcKindB256Z>
+        : kind == ESFM_KIND_B256 ? sweep_l2_tc_kernel<ESFM_KIND_B256> : sweep_l2_tc_kernel<ESFM_KIND_F32X64>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kern<<<grid, kTcThreads, smem, s>>>(p);

@@ -22,7 +22,7 @@
 //     (HMNMX2 / VHMNMX tournament, HFMA2.RELU threshold tests): ~1/2 the instructions per element of the fp32 epilogue.
 // The kernel is ROWS-ONLY: the cross-check is decided by finalize.cu from the row results (claims + histograms), and the train rows that
 // remain undecided are swept once more through this same kernel with the roles swapped and the query operand gathered
-// (SweepParams::gather).  Sweeps that need column minima (esfm_knn2_pair, $ESFM_TWO_PHASE=0) run on sweep_l2_tc.cu.
+// (SweepParams::gather).  Raw knn output (esfm_knn2_pair) needs column minima: it runs on sweep_l2_tc.cu.
 //
 // Pipeline: one persistent CTA per SM, 24 warps --
 //   warp 16      TMA producer: one cp.async.bulk per 36 KB train tile image into a 5-stage ring;

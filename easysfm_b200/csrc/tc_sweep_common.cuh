@@ -23,14 +23,11 @@ constexpr int kTcPartCols = kTile / kTcColParts;        // 32 columns per epilog
 constexpr int kTcStages = 3;                 // shared-memory train stages (68 KB each)
 constexpr int kTcThrBytes = kTile * 4;                  // 512: column thresholds riding with a train tile
 constexpr int kTcThrStages = 4;                         // threshold snapshots have their own (deeper) ring
-// "no bound yet" (also what cudaMemsetAsync writes into the column thresholds, hence a repeated byte): above every real value,
-// below the pad rows.  SURF: 7.4e28 (pads: 1e30).  ORB: 51015 (real 2 * hamming <= 512, pads >= 200704).  ORB "Z": 1.33e7 (keys < 2^24).
-constexpr uint32_t kTcBoundBitsF32 = 0x6f6f6f6fu, kTcBoundBitsB256 = 0x47474747u, kTcBoundBitsZ = 0x4b4b4b4bu;
 
 struct TcUnit {
     int pair, q_frame, t_frame;
     int nqt, ntt;
-    int qb0, qb1;        // query TILES [qb0, qb1) of this unit; walked in blocks of kTcQTiles
+    int qb0, qb1;        // query TILES [qb0, qb1) of this unit
 };
 
 __device__ __forceinline__ TcUnit tc_decode_unit(const SweepParams& p, int unit) {

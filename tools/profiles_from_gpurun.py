@@ -38,8 +38,8 @@ if os.path.exists(lp):
     traffic = {}
     for key, name, fin_grid, pairs, alg in (("surf_tc16", "sweep_win_kernel<0>", "(2368, 1, 1)", 2368, 8000 * (288 + 256)),
                                             ("orb_tc16", "sweep_win_kernel<1>", "(9472, 1, 1)", 9472, 4000 * (288 + 32)),
-                                            ("surf_tc", "sweep_l2_tc_kernel<1, 0>", "(2368, 1, 1)", 2368, 8000 * (544 + 256)),
-                                            ("orb_tc", "sweep_l2_tc_kernel<1, 2>", "(9472, 1, 1)", 9472, 4000 * (288 + 32)),
+                                            ("surf_tc", "sweep_l2_tc_kernel<0>", "(2368, 1, 1)", 2368, 8000 * (544 + 256)),
+                                            ("orb_tc", "sweep_l2_tc_kernel<2>", "(9472, 1, 1)", 9472, 4000 * (288 + 32)),
                                             ("surf", "sweep_l2_kernel", "(2368, 1, 1)", 2368, 8000 * 520),
                                             ("orb", "sweep_hamming_kernel", "(9472, 1, 1)", 9472, 4000 * 64)):
         g = [a for a, b in zip(L, L[1:]) if name in a["k"] and "finalize" in b["k"] and b["g"] == fin_grid]
