@@ -184,6 +184,47 @@ cudaError_t launch_pack_tch(const float* rows, const int* frame_rows, const int*
     return cudaGetLastError();
 }
 
+// F32X64 input range (esfm_bank_commit): per frame the largest |x| of any component, as float bits with the sign dropped (the integer
+// order of non-negative floats is their numeric order, so atomicMax works on them); an inf or NaN component leaves bits >= 0x7f800000.
+// One block per 128-row tile, one atomic per tile; frame_absmax must be zero on entry.
+__global__ void __launch_bounds__(256) frame_absmax_kernel(const float* __restrict__ rows, const int* __restrict__ frame_rows,
+                                                           const int* __restrict__ frame_row_off, const int* __restrict__ frame_tile_off,
+                                                           int n_frames, unsigned* __restrict__ frame_absmax) {
+    const int t = blockIdx.x;
+    int lo = 0, hi = n_frames - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (frame_tile_off[mid] <= t) lo = mid; else hi = mid - 1;
+    }
+    const int f = lo;
+    const int row0 = (t - frame_tile_off[f]) * kTile;
+    int valid = frame_rows[f] - row0;
+    valid = valid < 0 ? 0 : (valid > kTile ? kTile : valid);
+    const float4* src = reinterpret_cast<const float4*>(rows + ((size_t)frame_row_off[f] + row0) * kDim);
+    unsigned m = 0;
+    for (int idx = threadIdx.x; idx < valid * (kDim / 4); idx += blockDim.x) {
+        const float4 v = src[idx];
+        m = max(m, max(max(__float_as_uint(v.x) & 0x7fffffffu, __float_as_uint(v.y) & 0x7fffffffu),
+                       max(__float_as_uint(v.z) & 0x7fffffffu, __float_as_uint(v.w) & 0x7fffffffu)));
+    }
+    m = __reduce_max_sync(0xffffffffu, m);
+    __shared__ unsigned warp_max[8];
+    if ((threadIdx.x & 31) == 0) warp_max[threadIdx.x >> 5] = m;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < 8; ++w) m = max(m, warp_max[w]);
+        if (m) atomicMax(frame_absmax + f, m);
+    }
+}
+
+cudaError_t launch_frame_absmax(const float* rows, const int* frame_rows, const int* frame_row_off, const int* frame_tile_off, int n_frames,
+                                int n_tiles_total, unsigned* frame_absmax, cudaStream_t s) {
+    cudaError_t e = cudaMemsetAsync(frame_absmax, 0, (size_t)n_frames * sizeof(unsigned), s);
+    if (e != cudaSuccess || n_tiles_total <= 0) return e;
+    frame_absmax_kernel<<<n_tiles_total, 256, 0, s>>>(rows, frame_rows, frame_row_off, frame_tile_off, n_frames, frame_absmax);
+    return cudaGetLastError();
+}
+
 // B256 -> the FP8 tile images of tc_layout.cuh (Hamming on the tensor cores): one block per 128-row tile, one thread per
 // (row, 32-bit word): 32 bits -> 32 bytes of +-1.0 (E4M3), written as two 16-byte chunks into the SWIZZLE_128B atoms.
 __global__ void __launch_bounds__(256) pack_tc8_kernel(const uint32_t* __restrict__ rows, const int* __restrict__ frame_rows,

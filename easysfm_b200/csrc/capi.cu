@@ -7,6 +7,7 @@
 #include <sys/mman.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <new>
@@ -597,7 +598,7 @@ static int bank_alloc_layout(esfm_bank* b, bool adopt_mirror) {
     CUDA_TRY(cudaMemsetAsync((uint8_t*)b->d_rows + total_rows * b->row_bytes(), 0, (size_t)kHamTile * b->row_bytes(), ctx->stream));
     const size_t ne = (size_t)(b->n_frames + 1);
     if (!b->d_tables) {
-        cudaError_t e = pool_malloc(ctx, (void**)&b->d_tables, 3 * ne * sizeof(int));
+        cudaError_t e = pool_malloc(ctx, (void**)&b->d_tables, 4 * ne * sizeof(int));   // + per frame the largest |x| (bank_check_range)
         if (e != cudaSuccess) { cudaGetLastError(); return fail(ESFM_ERR_NOMEM, "cudaMallocAsync for the frame tables failed: %s", cudaGetErrorString(e)); }
         b->d_frame_rows = b->d_tables;
         b->d_row_off = b->d_tables + ne;
@@ -630,6 +631,35 @@ static void bank_release_staging(esfm_bank* b) {
     if (b->d_up && b->d_up != b->d_rows) cudaFreeAsync(b->d_up, ctx->stream);
     b->d_up = nullptr;
     b->up_cap = b->up_used = 0;
+}
+
+// F32X64: the input range of the committed rows (frame_absmax_kernel; set_frame_pinned and commit_device data never pass through host
+// staging, so it is measured on the device), which plan_sweep routes on.  Non-finite components, for which L2 matching has no defined answer,
+// and magnitudes beyond every engine's range are refused.
+static int bank_check_range(esfm_bank* b) {
+    if (b->kind != ESFM_KIND_F32X64) return ESFM_OK;
+    esfm_ctx* ctx = b->ctx;
+    const size_t ne = (size_t)(b->n_frames + 1);
+    unsigned* d_absmax = reinterpret_cast<unsigned*>(b->d_tables + 3 * ne);
+    CUDA_TRY(launch_frame_absmax((const float*)b->d_rows, b->d_frame_rows, b->d_row_off, b->d_tile_off, b->n_frames, b->tile_off[b->n_frames],
+                                 d_absmax, ctx->stream));
+    std::vector<unsigned> bits(b->n_frames);
+    CUDA_TRY(cudaMemcpyAsync(bits.data(), d_absmax, bits.size() * sizeof(unsigned), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    b->abs_max = 0.f;
+    b->frame_abs_min = INFINITY;
+    for (int f = 0; f < b->n_frames; ++f) {
+        if (b->rows[f] == 0) continue;
+        if (bits[f] >= 0x7f800000u) return fail(ESFM_ERR_INVALID, "frame %d has a non-finite (inf or NaN) component: L2 matching has no defined answer for it", f);
+        float m;
+        memcpy(&m, &bits[f], sizeof m);
+        if (m > kFfmaMaxAbs)
+            return fail(ESFM_ERR_INVALID, "frame %d has a component of magnitude %g; L2 matching supports |x| <= 2^59 (%g), where squared distances "
+                                          "stay finite in fp32", f, m, kFfmaMaxAbs);
+        b->abs_max = std::max(b->abs_max, m);
+        b->frame_abs_min = std::min(b->frame_abs_min, m);
+    }
+    return ESFM_OK;
 }
 
 extern "C" int esfm_bank_commit(esfm_bank_t* b) {
@@ -667,6 +697,7 @@ extern "C" int esfm_bank_commit(esfm_bank_t* b) {
     }
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));   // uploads done: pinned sources (ours and the caller's) are free again
     bank_release_staging(b);
+    if (int rc = bank_check_range(b)) return rc;
     b->committed = true;
     return ESFM_OK;
 }
@@ -685,6 +716,7 @@ extern "C" int esfm_bank_commit_device(esfm_bank_t* b) {
     if (int rc = set_device(b->ctx)) return rc;
     CUDA_TRY(cudaStreamSynchronize(b->ctx->stream));
     b->kmajor_built = b->tc_built = false;          // the raw rows may have been rewritten
+    if (int rc = bank_check_range(b)) return rc;
     b->committed = true;
     return ESFM_OK;
 }
@@ -777,6 +809,14 @@ struct SweepPlan {
     bool two_phase;      // Win cross-check: ratio test, then a verification sweep of the undecided train rows (finalize.cu)
 };
 
+// A SURF bank is swept by the context's engine when its components lie inside that engine's input range (esfm_internal.cuh), else by the
+// next engine that covers them: tc16 -> tc -> ffma (esfm_bank_commit has refused banks outside ffma's range).
+static int l2_engine_for(const esfm_bank* b, int engine) {
+    if (engine == ESFM_L2_ENGINE_TC16 && !(b->abs_max <= kTc16MaxAbs && b->frame_abs_min >= kTc16MinFrameAbs)) engine = ESFM_L2_ENGINE_TC;
+    if (engine == ESFM_L2_ENGINE_TC && !(b->abs_max <= kTcMaxAbs)) engine = ESFM_L2_ENGINE_FFMA;
+    return engine;
+}
+
 // The tc16 sweeps (sweep_win.cu) are ROWS-ONLY.  Their cross-check runs in TWO PHASES: (1) the rows-only sweep + ratio test, survivors
 // claim their train rows and histograms of every row's best / second-best value decide which survivors could still be beaten; (2) a
 // second rows-only sweep with the roles swapped over just the undecided train rows (gathered into the query operand), whose answer --
@@ -784,7 +824,7 @@ struct SweepPlan {
 // runs it on the fp32-accumulator sweep of sweep_l2_tc.cu (the bank's operand image is rebuilt on the switch).
 SweepPlan plan_sweep(const esfm_ctx* ctx, const esfm_bank* b, bool cross_check, bool knn) {
     const bool surf = b->kind == ESFM_KIND_F32X64;
-    const int engine = surf ? ctx->l2_engine : ctx->hamming_engine;
+    const int engine = surf ? l2_engine_for(b, ctx->l2_engine) : ctx->hamming_engine;
     SweepPlan s{};
     if (engine == (surf ? ESFM_L2_ENGINE_FFMA : ESFM_HAMMING_ENGINE_POPC)) {
         s.sweep = surf ? SweepKind::Ffma : SweepKind::Popc;

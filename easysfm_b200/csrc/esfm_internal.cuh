@@ -43,6 +43,18 @@ constexpr int kHamIdxBits = 20;                      // packed 32-bit key = dist
 // sweeps: SURF 7.4e28 (pads: 1e30), ORB 51015 (real 2 * hamming <= 512, pads >= 200704), ORB "Z" 1.33e7 (keys < 2^24).
 constexpr uint32_t kThrInit = 0x7f7f7f7fu;
 constexpr uint32_t kTcBoundBitsF32 = 0x6f6f6f6fu, kTcBoundBitsB256 = 0x47474747u, kTcBoundBitsZ = 0x4b4b4b4bu;
+// Input range of the SURF engines (DESIGN.md section 5.0, "Input range"): the largest |x| of any component, M, each sweep is correct for, with
+// D = kDim dims.  plan_sweep moves a bank outside an engine's range on to the next one (tc16 -> tc -> ffma); esfm_bank_commit refuses a bank
+// outside ffma's.  tc16: a = fp16(x) stays finite; below kTc16MinFrameAbs in some frame, fp16's subnormal step (2^-24, the split's absolute
+// error) is no longer small against that frame's distances.  tc: the largest 1/2 d^2 = 2 D M^2 = 2^95 stays below kTcBoundBitsF32 (7.4e28)
+// and the pad rows (kTcPadNorm, 1e30).  ffma: D (2M)^2 = 2^126 keeps finalize's direct-form sum finite, 1/2 d^2 <= 2^125 below kThrInit.
+constexpr float kTc16MaxAbs = 65504.f;
+constexpr float kTc16MinFrameAbs = 0x1p-6f;
+constexpr float kTcMaxAbs = 0x1p44f;
+constexpr float kFfmaMaxAbs = 0x1p59f;
+static_assert(2.0 * kDim * (double)kTcMaxAbs * kTcMaxAbs < 7.4e28 && 2.0 * kDim * (double)kFfmaMaxAbs * kFfmaMaxAbs < 3.39e38 &&
+                  kDim * 4.0 * kFfmaMaxAbs * kFfmaMaxAbs < (double)FLT_MAX,
+              "engine input ranges must stay below the column-threshold sentinels");
 // cudaMemsetAsync writes the thresholds' start value, so each sentinel must be one byte repeated
 __host__ __device__ constexpr bool is_byte_fill(uint32_t v) { return v == (v & 0xffu) * 0x01010101u; }
 static_assert(is_byte_fill(kThrInit) && is_byte_fill(kTcBoundBitsF32) && is_byte_fill(kTcBoundBitsB256) && is_byte_fill(kTcBoundBitsZ),
@@ -139,6 +151,8 @@ cudaError_t launch_pack_tc(const float* rows, const int* frame_rows, const int* 
                            int n_frames, int n_tiles_total, unsigned char* tc_main, cudaStream_t s);
 cudaError_t launch_pack_tch(const float* rows, const int* frame_rows, const int* frame_row_off, const int* frame_tile_off,
                             int n_frames, int n_tiles_total, unsigned char* tc_main, float* row_eps, float* frame_norm, cudaStream_t s);
+cudaError_t launch_frame_absmax(const float* rows, const int* frame_rows, const int* frame_row_off, const int* frame_tile_off, int n_frames,
+                                int n_tiles_total, unsigned* frame_absmax, cudaStream_t s);
 cudaError_t launch_sweep_l2(const SweepParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_sweep_win(const SweepParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_sweep_l2_tc(const SweepParams& p, int sm_count, cudaStream_t s);

@@ -142,6 +142,9 @@ struct esfm_bank {
     // host copies
     std::vector<int> row_off, tile_off;
     int max_rows = 0;
+    // F32X64, measured at commit: the largest |x| of any component, and the smallest of the non-empty frames' largest |x| (plan_sweep routes
+    // on both)
+    float abs_max = 0.f, frame_abs_min = 0.f;
     size_t row_bytes() const { return kind == ESFM_KIND_F32X64 ? esfm::kDim * sizeof(float) : 32; }
 };
 

@@ -3,6 +3,7 @@
 The fast sweep ranks with the query rounded to one fp16 term; rows its error bound cannot settle are re-swept exactly (the fallback
 sweep).  These tests build rows the fast values cannot settle -- near-ties at the ratio boundary, train rows a hair apart, duplicates,
 non-unit norms -- check the answers against oracle.match, that the fallback really ran, and that both modes return the same matches.
+Magnitudes outside tc16's input range (and the fallback at the smallest magnitude it keeps) are in test_gpu_input_range.py.
 """
 import os
 
