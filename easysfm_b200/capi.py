@@ -140,6 +140,10 @@ SIGNATURES = {
     "esfm_two_view_default_params": (c_int, [POINTER(TwoViewParams)]),
     "esfm_two_view_batch": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, POINTER(TwoViewParams), c_void_p, c_void_p]),
     "esfm_two_view_depth": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, POINTER(c_double), POINTER(c_int32)]),
+    "esfm_two_view_results": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, POINTER(TwoViewParams), c_int, POINTER(c_void_p),
+                                      c_void_p]),
+    "esfm_multi_two_view_results": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, POINTER(TwoViewParams), c_int,
+                                            POINTER(c_void_p), c_void_p]),
     "esfm_orb_extract": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_size_t, c_int, c_void_p, c_void_p, c_int, POINTER(c_int)]),
     "esfm_bank_set_frame_from_image": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_size_t, c_int, c_void_p, c_void_p, c_int, POINTER(c_int)]),
     "esfm_orb_last_timing": (c_int, [c_void_p, POINTER(c_double), POINTER(c_int)]),
@@ -701,6 +705,31 @@ class Results:
     def __iter__(self):
         for k in range(self.n_pairs):
             yield self.pair_at(k)
+
+    def verify(self, ctx_or_multi, keypoints, K, ransac_thre=1.0, ransac_prob=0.99, min_pair_matches=20, random_rate=20, seed=0, max_iters=1000):
+        """esfm_two_view_results (a Context) or esfm_multi_two_view_results (a MultiContext): the reference's estimate2D2D_E5P_RANSAC +
+        getDepthFast for every pair of this batch with more than min_pair_matches matches (sfm.cpp:163-166), on the device.
+        keypoints: one float32[n_f, 2] array of pixel coordinates per frame (frame_t::keypoints[k].pt); K: 3 x 3 (every frame) or
+        n_frames x 3 x 3 (a pair uses its query frame's).  Pair (i, j) draws its hypotheses from the key (i << 32) | j.
+        Returns (the inlier matches as a new Results in the same pair order, TWO_VIEW_DTYPE[n_pairs])."""
+        kps = [np.ascontiguousarray(k, np.float32).reshape(-1, 2) for k in keypoints]
+        kp_off = np.zeros(len(kps) + 1, np.int64)
+        kp_off[1:] = np.cumsum([len(k) for k in kps])
+        xy = np.concatenate(kps + [np.zeros((1, 2), np.float32)])
+        K = np.ascontiguousarray(K, np.float64)
+        k_per_frame = 1 if K.ndim == 3 else 0
+        if K.shape[-2:] != (3, 3) or (k_per_frame and K.shape[0] != len(kps)):
+            raise ValueError("K must be 3 x 3 or n_frames x 3 x 3")
+        prm = TwoViewParams()
+        _check(self._lib.esfm_two_view_default_params(ctypes.byref(prm)))
+        prm.ransac_thre, prm.ransac_prob, prm.seed = float(ransac_thre), float(ransac_prob), int(seed)
+        prm.max_iters, prm.random_rate = int(max_iters), int(random_rate)
+        out = np.zeros(max(self.n_pairs, 1), TWO_VIEW_DTYPE)
+        h = c_void_p()
+        fn = self._lib.esfm_multi_two_view_results if isinstance(ctx_or_multi, MultiContext) else self._lib.esfm_two_view_results
+        _check(fn(ctx_or_multi._h, self._h, len(kps), kp_off.ctypes.data, xy.ctypes.data, K.ctypes.data, k_per_frame, ctypes.byref(prm),
+                  int(min_pair_matches), ctypes.byref(h), out.ctypes.data))
+        return Results(self._lib, h), out[:self.n_pairs]
 
 
 class MultiContext:

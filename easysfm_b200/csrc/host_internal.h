@@ -5,6 +5,7 @@
 #include <condition_variable>
 #include <cstdarg>
 #include <cstdio>
+#include <cstdlib>
 #include <functional>
 #include <mutex>
 #include <string>
@@ -192,5 +193,35 @@ int orb_extract_impl(esfm_ctx* ctx, const unsigned char* image, int rows, int co
                      esfm_keypoint_t* keypoints, unsigned char* h_desc, int capacity, int* n_out, const OrbSink& sink);
 void orb_state_destroy(esfm_ctx* ctx);
 int reserve_stream_slots(esfm_ctx* ctx);     // allocate the pinned slots now (esfm_multi_init: outside any job's clock)
+
+// two_view.cu: verification of a results batch (esfm_two_view_results, esfm_multi_two_view_results).  The arguments of one call, checked once
+// by two_view_job, and what one device makes of its share of the batch's pairs.
+struct TvJob {
+    const esfm_results* matches = nullptr;
+    int n_frames = 0;
+    const int64_t* kp_off = nullptr;
+    const float* kp_xy = nullptr;
+    const double* K = nullptr;
+    int k_per_frame = 0;
+    esfm_two_view_params_t params{};
+    int min_pair_matches = 0;
+};
+struct TvShare {
+    std::vector<int64_t> ids;                        // batch positions of the share's pairs, ascending
+    std::vector<int32_t> counts;                     // inliers per pair
+    std::vector<uint64_t> offsets;                   // segment index << 40 | offset of the pair's inliers in `segments`
+    std::vector<esfm_results::Segment> segments;     // heap memory, one per chunk
+    std::vector<esfm_two_view_t> tv;
+    int64_t bad_pair = -1;                           // batch position of the first pair with a match index outside its frame's key points
+    TvShare() = default;
+    TvShare(const TvShare&) = delete;
+    TvShare& operator=(const TvShare&) = delete;
+    ~TvShare() { for (auto& s : segments) free(s.ptr); }
+};
+int two_view_job(const char* who, esfm_results* matches, int n_frames, const int64_t* kp_off, const float* kp_xy, const double* K, int k_per_frame,
+                 const esfm_two_view_params_t* params, int min_pair_matches, esfm_results_t** inliers, esfm_two_view_t* out, TvJob* job);
+int two_view_share(esfm_ctx* ctx, const TvJob& job, TvShare& share);
+// One results batch in the caller's pair order from the shares (their segments are adopted), and every pair's record to out.
+int two_view_assemble(const TvJob& job, std::vector<TvShare>& shares, esfm_results_t** inliers, esfm_two_view_t* out);
 
 }  // namespace esfm

@@ -374,3 +374,62 @@ extern "C" int esfm_multi_match_all_pairs(esfm_multi_bank_t* mb, double ratio, i
         }
     return esfm_multi_match_pairs(mb, pairs.data(), (int64_t)pairs.size(), ratio, cross_check, keep, out);
 }
+
+// ------------------------------------------------------------------------------------------------
+// verification of a results batch: deal pairs by match count, one worker thread per device, merge
+// ------------------------------------------------------------------------------------------------
+extern "C" int esfm_multi_two_view_results(esfm_multi_t* m, esfm_results_t* matches, int n_frames, const int64_t* kp_off, const float* kp_xy,
+                                           const double* K, int k_per_frame, const esfm_two_view_params_t* params, int min_pair_matches,
+                                           esfm_results_t** inliers, esfm_two_view_t* out) {
+    TvJob job;
+    if (int rc = two_view_job("esfm_multi_two_view_results", matches, n_frames, kp_off, kp_xy, K, k_per_frame, params, min_pair_matches, inliers, out, &job))
+        return rc;
+    if (!m) return fail(ESFM_ERR_INVALID, "esfm_multi_two_view_results: NULL argument");
+    DeviceRestore restore;
+    const double t0 = now_ms();
+    const int nd = m->n;
+    const int64_t n_pairs = (int64_t)matches->pairs.size();
+    // blocks of consecutive pairs to the least-loaded device, work = matches + 1 (the RANSAC of a pair scores every match)
+    std::vector<TvShare> shares((size_t)nd);
+    std::vector<double> load((size_t)nd, 0.0);
+    const int64_t block = std::max<int64_t>(1, std::min<int64_t>(kDealBlock, n_pairs / ((int64_t)nd * 8)));
+    for (int64_t b0 = 0; b0 < n_pairs; b0 += block) {
+        const int64_t b1 = std::min<int64_t>(n_pairs, b0 + block);
+        double w = 0.0;
+        for (int64_t k = b0; k < b1; ++k) w += (double)matches->counts[(size_t)k] + 1.0;
+        const int d = (int)(std::min_element(load.begin(), load.end()) - load.begin());
+        load[(size_t)d] += w;
+        for (int64_t k = b0; k < b1; ++k) shares[(size_t)d].ids.push_back(k);
+    }
+    const double mean = std::accumulate(load.begin(), load.end(), 0.0) / nd;
+    m->timing.work_imbalance = mean > 0 ? *std::max_element(load.begin(), load.end()) / mean - 1.0 : 0.0;
+    std::vector<int> rcs((size_t)nd, ESFM_OK);
+    std::vector<std::string> errs((size_t)nd);
+    std::vector<double> dev_ms((size_t)nd, 0.0);
+    auto work = [&](int d) {
+        const double s0 = now_ms();
+        rcs[(size_t)d] = two_view_share(m->ctx[(size_t)d], job, shares[(size_t)d]);
+        if (rcs[(size_t)d]) errs[(size_t)d] = g_last_error;      // (the message lives in the worker's thread-local slot)
+        dev_ms[(size_t)d] = now_ms() - s0;
+    };
+    if (nd == 1) {
+        work(0);
+    } else {
+        std::vector<std::thread> threads;
+        for (int d = 0; d < nd; ++d) threads.emplace_back(work, d);
+        for (auto& t : threads) t.join();
+    }
+    // the first offending pair of the batch, else the first failing device
+    int failed = -1;
+    for (int d = 0; d < nd; ++d) {
+        if (!rcs[(size_t)d]) continue;
+        const int64_t b = shares[(size_t)d].bad_pair, fb = failed < 0 ? -1 : shares[(size_t)failed].bad_pair;
+        if (failed < 0 || (b >= 0 && (fb < 0 || b < fb))) failed = d;
+    }
+    if (failed >= 0) return fail(rcs[(size_t)failed], "device slot %d (cuda:%d): %s", failed, m->devices[(size_t)failed], errs[(size_t)failed].c_str());
+    const int rc = two_view_assemble(job, shares, inliers, out);
+    m->timing.match_ms = now_ms() - t0;
+    m->timing.device_ms_max = *std::max_element(dev_ms.begin(), dev_ms.end());
+    m->timing.device_ms_min = *std::min_element(dev_ms.begin(), dev_ms.end());
+    return rc;
+}

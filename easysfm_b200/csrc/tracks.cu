@@ -179,8 +179,8 @@ extern "C" int esfm_tracks_finish_frame(esfm_tracks_t* t, int frame_i) {
 
 // The whole pair loop of sfm.cpp:140-217 over a batch that holds all pairs in the reference's order.  Pairs with at most
 // `min_pair_matches` matches contribute nothing (sfm.cpp:163: `if (temp_matches.size() > num_min_pair)`, 20 in the reference);
-// the others contribute ALL their matches -- the reference first thins them with the 5-point RANSAC of estimate_motion.cpp:27-97,
-// which is not part of this library (a caller that has inliers feeds them with esfm_tracks_add_pair instead).
+// the others contribute ALL their matches.  The reference feeds the inliers of its 5-point RANSAC (estimate_motion.cpp:27-97): that is
+// this loop over the batch esfm_two_view_results returns (pairs at or below 20 matches have no inliers there) with min_pair_matches = 0.
 extern "C" int esfm_tracks_build(esfm_tracks_t* t, esfm_results_t* r, int min_pair_matches) {
     if (!t || !r) return fail(ESFM_ERR_INVALID, "esfm_tracks_build: NULL argument");
     if (t->frames_done != 0) return fail(ESFM_ERR_STATE, "tracks already (partly) built");

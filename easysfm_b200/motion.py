@@ -1,6 +1,8 @@
 """Python mirror of the reference's MotionEstimator for the two-view step (cpp_code/include/estimate_motion.h:17-20, :33-34;
 cpp_code/src/estimate_motion.cpp:27-97, :234-283), on the GPU through esfm_two_view_batch.  Same names and argument meaning as the reference;
-the batch form serves the all-pairs loop of cpp_code/test/sfm.cpp:140-166 in one call."""
+the batch form serves the all-pairs loop of cpp_code/test/sfm.cpp:140-166 in one call.  For a match batch (capi.Results) the same step runs
+without gathering on the host: Results.verify returns the inlier matches as a new batch plus a pose per pair, keyed like this class's per-pair
+calls when pair_id = (frame_1 << 32) | frame_2."""
 from __future__ import annotations
 
 import numpy as np

@@ -14,6 +14,9 @@
 //   * resume: p3dv::esfm_save_matches(path) after the prepare step writes the whole batch to a match file;
 //     p3dv::esfm_load_matches(frames, 'S'|'O', ratio, path) in a later run makes the same lookups work without
 //     matching again (and without touching the GPU).
+//   * verification: p3dv::esfm_verify_all_pairs(frames, ransac_thre, ransac_prob, num_min_pair) after the prepare (or load) step
+//     verifies every pair of the batch on the device (esfm_two_view_results; ESFM_GPUS=N > 1: on N GPUs); later
+//     MotionEstimator::estimate2D2D_E5P_RANSAC calls with a pair's unaltered matches are lookups (estimate_motion_gpu.cpp).
 //
 // Semantics kept from the reference: matches are APPENDED (push_back, :90/:135), ascending queryIdx, imgIdx = 0,
 // returns true; ratio test in double (:88/:133); the stdout summary lines (:81,96-97 / :126,141-142).
@@ -32,6 +35,7 @@
 
 #include "feature_matching.h"  // EasySFM's own header: class p3dv::FeatureMatching, frame_t
 #include "esfm_match.h"
+#include "esfm_verified.h"
 
 namespace p3dv {
 namespace {
@@ -151,6 +155,7 @@ bool match_common(esfm_kind kind, const char* tag, frame_t& f1, frame_t& f2, std
 bool esfm_prepare_all_pairs(std::vector<frame_t>& frames, char feature, double ratio_thre, bool cross_check) {
     GpuState& s = state();
     const int gpus = env_gpus();
+    esfm_shim::verified().clear();
     if (s.results) { esfm_results_destroy(s.results); s.results = nullptr; }
     if (s.mbank) { esfm_multi_bank_destroy(s.mbank); s.mbank = nullptr; }
     if (s.bank) { esfm_bank_destroy(s.bank); s.bank = nullptr; }
@@ -218,6 +223,7 @@ bool esfm_load_matches(std::vector<frame_t>& frames, char feature, double ratio_
         esfm_results_destroy(r);
         return false;
     }
+    esfm_shim::verified().clear();
     if (s.results) esfm_results_destroy(s.results);
     s.results = r;
     s.kind = want;
@@ -226,6 +232,70 @@ bool esfm_load_matches(std::vector<frame_t>& frames, char feature, double ratio_
     s.have_mode = true;
     s.frame_index.clear();
     for (size_t i = 0; i < frames.size(); ++i) s.frame_index[frames[i].frame_id] = (int)i;
+    return true;
+}
+
+// The two-view step of the reference's loop (sfm.cpp:163-166: estimate2D2D_E5P_RANSAC on every pair with more than num_min_pair matches) for
+// the whole prepared or loaded batch at once, on the device.  A frame's key points are frame_t::keypoints, its camera frame_t::K_cam (a pair
+// uses its query frame's, as estimate_motion.cpp:43 does).  Frame ids must be the frames' positions, as the reference numbers them: the
+// per-call path keys each pair's RANSAC samples by its frame ids, the batch by its positions, and the lookups rely on the two being equal.
+bool esfm_verify_all_pairs(std::vector<frame_t>& frames, double ransac_thre, double ransac_prob, int num_min_pair) {
+    GpuState& s = state();
+    esfm_shim::VerifiedBatch& v = esfm_shim::verified();
+    v.clear();
+    if (!s.results) { std::cerr << "esfm_verify_all_pairs: call esfm_prepare_all_pairs or esfm_load_matches first" << std::endl; return false; }
+    const int n = (int)frames.size();
+    std::vector<int64_t> kp_off((size_t)n + 1, 0);
+    for (int i = 0; i < n; ++i) {
+        if (frames[(size_t)i].frame_id != (unsigned)i) {
+            std::cerr << "esfm_verify_all_pairs: frame " << i << " has frame_id " << frames[(size_t)i].frame_id << " (ids must be 0..n-1)" << std::endl;
+            return false;
+        }
+        kp_off[(size_t)i + 1] = kp_off[(size_t)i] + (int64_t)frames[(size_t)i].keypoints.size();
+    }
+    std::vector<float> xy((size_t)kp_off[(size_t)n] * 2 + 2);
+    std::vector<double> K((size_t)n * 9 + 9);
+    for (int i = 0; i < n; ++i) {
+        const frame_t& f = frames[(size_t)i];
+        for (size_t k = 0; k < f.keypoints.size(); ++k) {
+            xy[2 * ((size_t)kp_off[(size_t)i] + k)] = f.keypoints[k].pt.x;
+            xy[2 * ((size_t)kp_off[(size_t)i] + k) + 1] = f.keypoints[k].pt.y;
+        }
+        for (int r = 0; r < 3; ++r)
+            for (int c = 0; c < 3; ++c) K[(size_t)i * 9 + 3 * r + c] = (double)f.K_cam(r, c);
+    }
+    esfm_two_view_params_t prm;
+    esfm_two_view_default_params(&prm);
+    prm.ransac_thre = ransac_thre;
+    prm.ransac_prob = ransac_prob;
+    prm.seed = esfm_shim::ransac_seed();
+    int64_t n_pairs = 0;
+    esfm_results_counts(s.results, &n_pairs, nullptr);
+    v.tv.resize((size_t)std::max<int64_t>(n_pairs, 1));
+    const int gpus = env_gpus();
+    int rc = ESFM_OK;
+    if (gpus > 1) {
+        if (!s.multi) rc = esfm_multi_init(gpus, nullptr, &s.multi);
+        if (rc == ESFM_OK)
+            rc = esfm_multi_two_view_results(s.multi, s.results, n, kp_off.data(), xy.data(), K.data(), 1, &prm, num_min_pair, &v.inliers, v.tv.data());
+    } else {
+        if (!ensure_ctx()) return false;
+        rc = esfm_two_view_results(s.ctx, s.results, n, kp_off.data(), xy.data(), K.data(), 1, &prm, num_min_pair, &v.inliers, v.tv.data());
+    }
+    if (rc != ESFM_OK) {
+        std::cerr << "esfm_verify_all_pairs failed: " << esfm_last_error() << std::endl;
+        v.clear();
+        return false;
+    }
+    v.matches = s.results;
+    v.ransac_thre = ransac_thre;
+    v.ransac_prob = ransac_prob;
+    v.min_pair = num_min_pair;
+    for (int64_t k = 0; k < n_pairs; ++k) {
+        int q = 0, t = 0;
+        esfm_results_pair_at(s.results, k, &q, &t, nullptr, nullptr);
+        v.index.emplace(((uint64_t)(uint32_t)q << 32) | (uint32_t)t, k);
+    }
     return true;
 }
 

@@ -266,9 +266,10 @@ int esfm_tracks_destroy(esfm_tracks_t* tracks);
 int esfm_tracks_add_pair(esfm_tracks_t* tracks, int frame_i, int frame_j, const esfm_dmatch_t* inlier_matches, int n);
 /* End of frame_i's row: fresh ids for its unlabelled keypoints, its row of the track matrix (sfm.cpp:199-213). */
 int esfm_tracks_finish_frame(esfm_tracks_t* tracks, int frame_i);
-/* The whole loop over a batch holding all pairs in loop order (esfm_match_all_pairs / esfm_multi_match_all_pairs): pairs with
- * more than min_pair_matches matches (sfm.cpp:163: 20) contribute all their matches -- the reference first thins them with its
- * 5-point RANSAC (estimate_motion.cpp:27-97), which this library does not replace. */
+/* The whole loop over a batch holding all pairs in loop order: pairs with more than min_pair_matches matches contribute all of them.
+ * The reference feeds each pair's RANSAC inliers (sfm.cpp:163-194), so its tracks come from the verified batch of
+ * esfm_two_view_results (pairs at or below 20 matches already have no inliers there) with min_pair_matches = 0; a matched batch
+ * (esfm_match_all_pairs / esfm_multi_match_all_pairs) with min_pair_matches = 20 gives the tracks of unverified matches. */
 int esfm_tracks_build(esfm_tracks_t* tracks, esfm_results_t* results, int min_pair_matches);
 /* frame_t::unique_pixel_ids / unique_pixel_has_match of one frame (library-owned, n = its keypoints). */
 int esfm_tracks_frame(esfm_tracks_t* tracks, int frame, const int32_t** unique_pixel_ids, const uint8_t** unique_pixel_has_match, int* n);
@@ -301,10 +302,10 @@ typedef struct esfm_multi_bank esfm_multi_bank_t;
 typedef struct esfm_multi_timing_t {
     double broadcast_ms;      /* last esfm_multi_bank_commit: replication of the raw bank on devices 1..n-1 (host wall clock) */
     double commit_ms;         /* last esfm_multi_bank_commit: the whole call */
-    double match_ms;          /* last esfm_multi_match_*: the whole call (host wall clock, results merged) */
+    double match_ms;          /* last esfm_multi_match_* or esfm_multi_two_view_results: the whole call (host wall clock, results merged) */
     double device_ms_max;     /* ... slowest device's share */
     double device_ms_min;     /* ... fastest device's share */
-    double work_imbalance;    /* max over devices of assigned comparisons / mean, minus 1 */
+    double work_imbalance;    /* max over devices of assigned comparisons (verification: matches) / mean, minus 1 */
     int used_nccl;            /* 1 = ncclBroadcast, 0 = device copies (one device, or a device listed twice) */
 } esfm_multi_timing_t;
 
@@ -366,6 +367,28 @@ int esfm_two_view_batch(esfm_ctx_t* ctx, int64_t n_pairs, const int64_t* pair_of
  * points in baseline lengths, *n_used (optional) = how many were triangulated. */
 int esfm_two_view_depth(esfm_ctx_t* ctx, int64_t n_matches, const float* pts1, const float* pts2, const double* K, const double* R,
                         const double* t, int random_rate, double* depth, int32_t* n_used);
+/* Verification of a whole match batch, the step between matching and track building in the reference's loop (sfm.cpp:163-194).
+ * `matches` is a fetched batch (ESFM_KEEP_MATCHES; a digests-only or unfetched device-resident batch -> ESFM_ERR_STATE), matched in this run
+ * or loaded with esfm_results_load.  Key points: frame f owns kp_xy[2*k], kp_xy[2*k+1] for k in [kp_off[f], kp_off[f+1])
+ * (frame_t::keypoints[k].pt), n_frames + 1 offsets from kp_off[0] = 0.  K: one row-major 3 x 3 for all frames (k_per_frame = 0) or one per
+ * frame; a pair uses its QUERY frame's K (estimate_motion.cpp:43).  Pairs with <= min_pair_matches matches are not verified (sfm.cpp:163, 20
+ * in the reference): ok = 0, no inliers, iters = 0.  Pair (i, j) draws its hypotheses from the key (i << 32) | j with params->seed -- the key
+ * the C++ drop-in uses per call -- so its result does not depend on the batch, its position in it, or the device; params->first_pair must
+ * be 0.  Key-point gathering, RANSAC, pose and inlier compaction run on the device; only inlier records and results return.
+ * *inliers: a new batch with the same pairs in the same order, each pair's inlier records unchanged and in their original order
+ * (estimate_motion.cpp:54-60), kind / ratio / cross_check / frame rows copied from `matches`; out: one record per pair.
+ * ESFM_ERR_INVALID, before any output: NULL arguments, a pair outside [0, n_frames), stored frame rows (a version-2 file, or any batch the
+ * library matched) that differ from the key-point counts, bad parameters (as esfm_two_view_batch), or a queryIdx / trainIdx outside its
+ * frame's key points (found on the device; the message names the first such pair). */
+int esfm_two_view_results(esfm_ctx_t* ctx, esfm_results_t* matches, int n_frames, const int64_t* kp_off, const float* kp_xy, const double* K,
+                          int k_per_frame, const esfm_two_view_params_t* params, int min_pair_matches, esfm_results_t** inliers,
+                          esfm_two_view_t* out);
+/* The same on the devices of `multi`: consecutive blocks of pairs are dealt to the devices by match count, each device verifies its share with
+ * its own copy of the key points, the shares are merged in the batch's pair order.  Byte-identical to esfm_two_view_results at any device
+ * count (the keys are frame ids). */
+int esfm_multi_two_view_results(esfm_multi_t* multi, esfm_results_t* matches, int n_frames, const int64_t* kp_off, const float* kp_xy,
+                                const double* K, int k_per_frame, const esfm_two_view_params_t* params, int min_pair_matches,
+                                esfm_results_t** inliers, esfm_two_view_t* out);
 
 /* ---- ORB extraction: the step before the path (SURVEY.md section 8(f) rank 4) -------------------------------------------------------------
  * Replaces FeatureMatching::detectFeaturesORB (cpp_code/src/feature_matching.cpp:14-41; decl cpp_code/include/feature_matching.h:13, called
