@@ -49,6 +49,7 @@ class Stats(ctypes.Structure):
         ("sweep_ms_total", c_double),
         ("sweep_launches", c_uint64),
         ("fallback_rows", c_uint64),
+        ("verified_rows", c_uint64),
     ]
 
     def as_dict(self):

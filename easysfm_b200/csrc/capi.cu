@@ -295,7 +295,7 @@ extern "C" int esfm_init(int device, void* cuda_stream, esfm_ctx_t** out) {
             e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
             if (e != cudaSuccess) return bail(ESFM_ERR_CUDA, "cudaEventCreate", e);
         }
-        e = cudaMalloc((void**)&cb.d_cursor, 3 * sizeof(unsigned long long));
+        e = cudaMalloc((void**)&cb.d_cursor, 4 * sizeof(unsigned long long));
         if (e != cudaSuccess) return bail(ESFM_ERR_NOMEM, "cudaMalloc", e);
     }
     {   // banks come and go (one per all-pairs call in the per-call API): they are allocated stream-ordered from a memory pool
@@ -895,7 +895,7 @@ int ensure_scratch(esfm_ctx* ctx, const esfm_bank* b, const SweepPlan& sw, const
             cb.pairs_cap = pl.chunk_pairs;
         }
         if (int rc = grow_pinned(&cb.h_pairs, &cb.h_pairs_cap, pl.chunk_pairs)) return rc;
-        const size_t meta = pl.chunk_pairs * (sizeof(int32_t) + sizeof(unsigned long long)) + 3 * sizeof(unsigned long long);
+        const size_t meta = pl.chunk_pairs * (sizeof(int32_t) + sizeof(unsigned long long)) + 4 * sizeof(unsigned long long);
         if (int rc = grow_pinned(&cb.h_meta, &cb.h_meta_bytes, meta)) return rc;
     }
     return ESFM_OK;
@@ -963,7 +963,7 @@ int units_per_pair(const esfm_ctx* ctx, const esfm_bank* b, const SweepPlan& sw,
 int run_chunk(esfm_ctx* ctx, esfm_bank* b, const SweepPlan& sw, const ChunkPlan& pl, ChunkBuf& cb, size_t n, double ratio, int cross_check,
               int32_t* knn_idx, float* knn_dist) {
     CUDA_TRY(cudaMemsetAsync(ctx->keys, (int)(kKeyInit & 0xff), n * 4 * (size_t)pl.stride * sizeof(u64), ctx->stream));
-    CUDA_TRY(cudaMemsetAsync(cb.d_cursor, 0, 3 * sizeof(unsigned long long), ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(cb.d_cursor, 0, 4 * sizeof(unsigned long long), ctx->stream));
     if (sw.sweep == SweepKind::Tc || sw.sweep == SweepKind::Win) { if (int rc = ensure_tc_layout(ctx, b, sw.image)) return rc; }
     else if (sw.sweep == SweepKind::Ffma) { if (int rc = ensure_kmajor_layout(ctx, b)) return rc; }
     if (sw.thr_fill >= 0)
@@ -1009,6 +1009,7 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const SweepPlan& sw, const ChunkPlan&
     fp.phase = sw.two_phase ? 1 : 0;
     fp.gather = reinterpret_cast<int*>(ctx->col_thr);
     fp.gather_cnt = ctx->gather_cnt;
+    fp.verified_rows = cb.d_cursor + 3;
     fp.arena = cb.arena;
     fp.arena_cap = cb.arena_cap;
     fp.cursor = cb.d_cursor;
@@ -1017,10 +1018,10 @@ int run_chunk(esfm_ctx* ctx, esfm_bank* b, const SweepPlan& sw, const ChunkPlan&
     fp.pair_cnt = cb.d_pair_cnt;
     fp.knn_idx = knn_idx;
     fp.knn_dist = knn_dist;
+    if (sw.sweep == SweepKind::Win && b->kind == ESFM_KIND_F32X64) fp.frame_norm = tch_frame_norm(b);   // (phase 1's margin, both modes)
     if (sw.fast) {
         // rows the fast sweep cannot settle -> the pair's gather list -> one exact sweep of just those rows (sweep time)
         fp.row_eps = tch_row_eps(b);
-        fp.frame_norm = tch_frame_norm(b);
         fp.fallback_rows = cb.d_cursor + 2;
         e = launch_win_classify(fp, ctx->stream);
         if (e != cudaSuccess) return fail(ESFM_ERR_CUDA, "fast-sweep classification kernel launch failed: %s", cudaGetErrorString(e));
@@ -1172,13 +1173,13 @@ int esfm::match_pairs_impl(esfm_bank* b, const esfm_pair_t* pairs, int64_t n_pai
         ChunkBuf& cb = ctx->buf[k & 1];
         CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, cb.ev_t2, 0));
         unsigned long long* h_cur = (unsigned long long*)cb.h_meta;
-        unsigned long long* h_off = h_cur + 3;
+        unsigned long long* h_off = h_cur + 4;
         int32_t* h_cnt = (int32_t*)(h_off + ch.n);
-        CUDA_TRY(cudaMemcpyAsync(h_cur, cb.d_cursor, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->copy_stream));
+        CUDA_TRY(cudaMemcpyAsync(h_cur, cb.d_cursor, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->copy_stream));
         CUDA_TRY(cudaMemcpyAsync(h_off, cb.d_pair_off, ch.n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->copy_stream));
         CUDA_TRY(cudaMemcpyAsync(h_cnt, cb.d_pair_cnt, ch.n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->copy_stream));
         CUDA_TRY(cudaEventRecord(cb.ev_meta, ctx->copy_stream));
-        ctx->stats.d2h_bytes += ch.n * (sizeof(int32_t) + sizeof(unsigned long long)) + 3 * sizeof(unsigned long long);
+        ctx->stats.d2h_bytes += ch.n * (sizeof(int32_t) + sizeof(unsigned long long)) + 4 * sizeof(unsigned long long);
         return ESFM_OK;
     };
     auto finish = [&](size_t k) -> int {            // chunk k has been finalised: book its pairs, bring its matches to the host
@@ -1187,11 +1188,12 @@ int esfm::match_pairs_impl(esfm_bank* b, const esfm_pair_t* pairs, int64_t n_pai
         CUDA_TRY(cudaEventSynchronize(cb.ev_meta));
         if (int rc = collect_timing(ctx, cb)) return rc;
         const unsigned long long* h_cur = (const unsigned long long*)cb.h_meta;
-        const unsigned long long* h_off = h_cur + 3;
+        const unsigned long long* h_off = h_cur + 4;
         const int32_t* h_cnt = (const int32_t*)(h_off + ch.n);
         const unsigned long long n_matches = h_cur[0];
         if ((int)h_cur[1] != 0 || n_matches > cb.arena_cap) return fail(ESFM_ERR_CAPACITY, "match arena overflow (internal sizing error)");
         ctx->stats.fallback_rows += h_cur[2];
+        ctx->stats.verified_rows += h_cur[3];
         const int seg = (int)res->segments.size();
         for (size_t i = 0; i < ch.n; ++i) {
             res->counts[ch.c0 + ch.order[i]] = h_cnt[i];

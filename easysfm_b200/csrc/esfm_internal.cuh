@@ -134,9 +134,11 @@ struct FinalizeParams {
     int* gather_cnt;            // [n_pairs]
     // SURF rows from the FAST sweep (SweepParams::win_fast; NULL = every row was swept in exact mode): per bank row |x - fp16(x)|_2,
     // per frame the largest |x|_2 (launch_pack_tch) -> win_fast_eps.  Rows whose key carries kWinExactMark were re-swept exactly.
+    // frame_norm is also set in exact mode: phase 1 of the two-phase cross-check scales its margin with it.
     const float* row_eps;
     const float* frame_norm;
     unsigned long long* fallback_rows;   // win_classify: += rows put on the fallback list
+    unsigned long long* verified_rows;   // two-phase cross-check, phase 1: += train rows put on the verification list
     // optional raw knn output for one pair (esfm_knn2_pair)
     int32_t* knn_idx;
     float* knn_dist;

@@ -442,14 +442,23 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
         // survivors: beaten by another survivor -> dropped; below every possible rival -> decided (state 1); else its train row goes on
         // the pair's list for the verification sweep (state 2; any order: the slot is looked up through ck1)
         int* gl = p.gather + (size_t)pair * p.stride;
+        // SURF: the histograms hold the sweep's 1/2 d^2, whose error grows with the magnitudes the expansion form cancels,
+        // m = 1/2 (nq^2 + nt^2) + nq nt (nq, nt: the frames' largest row norms, as in win_fast_eps) -- at norm 64 one ulp of a half norm
+        // alone is 2.4e-4.  Compare with a margin of 2^-14 m (twice the rounding term win_fast_eps allows the 9-slot sweep; the exact
+        // sweep has 13 slots), at least 1e-5.  Fast-mode rows entered the histograms at value - e already; the margin covers the rows
+        // swept in exact mode (e = 0).  A larger margin only sends more train rows to the verification sweep.
+        float margin = 1e-5f;
+        if (KIND == ESFM_KIND_F32X64 && p.frame_norm) {
+            const float nq = p.frame_norm[pd.q_frame], nt = p.frame_norm[pd.t_frame];
+            margin = fmaxf(margin, 0x1p-14f * (0.5f * (nq * nq + nt * nt) + nq * nt));
+        }
         for (int q = threadIdx.x; q < fq; q += kFinThreads) {
             const u64 v = rk1[q];
             if (v == kKeyInit) continue;
             const int t1 = (int)(uint32_t)v;
             const float d1 = __uint_as_float((uint32_t)(v >> 32));
             if (ck1[t1] != make_key((uint32_t)(v >> 32), (uint32_t)q)) { rk1[q] = kKeyInit; continue; }
-            // (SURF: the histograms hold sweep-form 1/2 d^2, within ~1e-6 of the direct form: compare with a margin)
-            const float mine_v = KIND == ESFM_KIND_B256 ? 2.f * d1 : 0.5f * d1 * d1 + 1e-5f;
+            const float mine_v = KIND == ESFM_KIND_B256 ? 2.f * d1 : 0.5f * d1 * d1 + margin;
             if (s_hist[0][fin_bucket<KIND>(mine_v)] == 0u) { rk2[q] = 1; continue; }
             const unsigned int slot = atomicAdd(&s_targets, 1u);
             gl[slot] = t1;
@@ -457,7 +466,10 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const FinalizePar
             rk2[q] = 2;
         }
         __syncthreads();
-        if (threadIdx.x == 0) p.gather_cnt[pair] = (int)s_targets;
+        if (threadIdx.x == 0) {
+            p.gather_cnt[pair] = (int)s_targets;
+            if (s_targets) atomicAdd(p.verified_rows, (unsigned long long)s_targets);
+        }
         return;
     }
     // block total -> one arena allocation per pair

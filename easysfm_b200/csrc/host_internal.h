@@ -55,7 +55,8 @@ struct ChunkBuf {
     unsigned long long* d_pair_off = nullptr;
     int32_t* d_pair_cnt = nullptr;
     size_t pairs_cap = 0;
-    unsigned long long* d_cursor = nullptr;      // [0] arena cursor, [1] overflow flag, [2] rows re-swept by the SURF fallback sweep
+    unsigned long long* d_cursor = nullptr;      // [0] arena cursor, [1] overflow flag, [2] rows re-swept by the SURF fallback sweep,
+                                                 // [3] train rows put on the verification sweep's gather lists
     esfm_dmatch_t* arena = nullptr;              // dense match arena of the chunk
     size_t arena_cap = 0;                        // in matches
     uint64_t generation = 0;                     // bumped whenever the arena is overwritten

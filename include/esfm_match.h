@@ -86,6 +86,7 @@ typedef struct esfm_stats_t {
     double sweep_ms_total;     /* sum of sweep kernel device times */
     uint64_t sweep_launches;   /* number of sweep kernel launches */
     uint64_t fallback_rows;    /* SURF tc16: query rows the 9-slot sweep could not settle, re-swept in exact (13-slot) mode */
+    uint64_t verified_rows;    /* tc16 cross-check: train rows the ratio-test histograms could not decide, re-swept by the verification sweep */
 } esfm_stats_t;
 
 int esfm_abi_version(void);
